@@ -1,8 +1,8 @@
 """Benchmark of the hot path: contrastive fwd+bwd pairs/sec @ global batch 65536, d=512, bf16.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n 65536] [--d 512]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n 65536] [--d 512] [--dump-outputs DIR]
 
-One JSON line on rank 0 (see the task contract): `value` = pairs/s with inputs resident in HBM,
+One JSON line on rank 0: `value` = pairs/s with inputs resident in HBM,
 `e2e` = the same through the public API from pinned HOST buffers (H2D of the embeddings + D2H of the
 loss inside the timed region), `roofline` for the dominant kernel (tcgen05 backward side), and a
 `cpu_baseline` (the reference's op sequence on the box's host cores, bounded sample).
@@ -177,6 +177,43 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+def gathered(x, group, world):
+    """The row shards of every rank, concatenated in rank order (NCCL, untimed); `x` itself on one GPU."""
+    if world == 1:
+        return x
+    import torch
+    import torch.distributed as dist
+    out = torch.empty((world * x.shape[0],) + tuple(x.shape[1:]), dtype=x.dtype, device=x.device)
+    dist.all_gather_into_tensor(out, x.contiguous(), group=group)
+    return out
+
+
+# ------------------------------------------------------------------------------------------------ outputs
+DUMP_GRAD_BYTES = 32 << 20     # --dump-outputs: the two gradient arrays together, as float32
+
+
+def dump_outputs(out_dir, outs, group, rank, world):
+    """--dump-outputs: what the timed step returns to its caller -- loss, d_a, d_b, d_logit_scale -- as float32 .npy files
+    in `out_dir`, so that two builds can be compared output for output (the inputs are seeded).  Gradients of every
+    rank are gathered to rank 0; above DUMP_GRAD_BYTES a fixed, seeded sample of global rows is written (`rows.npy`,
+    float64, holds their indices)."""
+    import numpy as np
+    import torch
+    loss, da, db, dls = outs
+    da, db = gathered(da, group, world), gathered(db, group, world)
+    if rank != 0:
+        return
+    n, d = da.shape
+    k = min(n, DUMP_GRAD_BYTES // (2 * 4 * d))
+    rows = np.arange(n) if k == n else np.sort(np.random.default_rng(20261020).choice(n, size=k, replace=False))
+    idx = torch.as_tensor(rows, device=da.device)
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss, "d_a": da[idx], "d_b": db[idx], "d_logit_scale": dls}
+    for name, x in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), x.detach().float().cpu().numpy())
+    np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------------------ parity
 def parity_check(step_fn, a, b, logit_scale, group, rank, world, n_rows_sample):
     """One extra step OUTSIDE the timed region, compared with the sampled-row CPU oracle (oracle/sampled.py) at the
@@ -186,18 +223,9 @@ def parity_check(step_fn, a, b, logit_scale, group, rank, world, n_rows_sample):
     shards.  -> the `parity` dict on rank 0, None elsewhere."""
     import numpy as np
     import torch
-    import torch.distributed as dist
     loss, da, db, dls = step_fn()
     torch.cuda.synchronize()
-
-    def gathered(x):
-        if world == 1:
-            return x
-        out = torch.empty((world * x.shape[0],) + tuple(x.shape[1:]), dtype=x.dtype, device=x.device)
-        dist.all_gather_into_tensor(out, x.contiguous(), group=group)
-        return out
-
-    a_all, b_all, da_all, db_all = gathered(a), gathered(b), gathered(da), gathered(db)
+    a_all, b_all, da_all, db_all = (gathered(x, group, world) for x in (a, b, da, db))
     if rank != 0:
         return None
     from oracle import sampled as SO
@@ -398,10 +426,11 @@ def run_ours(args, rank, local_rank, world):
     loss_host = torch.empty((), dtype=torch.float32).pin_memory()
 
     def step_resident():
+        # logit_scale.grad accumulates over the steps of a run (nothing clears it), as in a loop without zero_grad
         ar, br = a.detach().requires_grad_(True), b.detach().requires_grad_(True)
         loss = fused_clip_loss(ar, br, logit_scale, group=group, engine=eng)
         loss.backward()
-        return loss
+        return loss.detach(), ar.grad, br.grad, logit_scale.grad
 
     def step_e2e():
         ar = a_host.to(dev, non_blocking=True).requires_grad_(True)
@@ -417,11 +446,12 @@ def run_ours(args, rank, local_rank, world):
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """-> (ms for `steps` calls of fn, what the last call returned)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
@@ -429,7 +459,7 @@ def run_ours(args, rank, local_rank, world):
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t)
-        return ms
+        return ms, out
 
     for _ in range(max(args.warmup, 3)):
         step_resident()
@@ -450,7 +480,7 @@ def run_ours(args, rank, local_rank, world):
                     f.write(f"{(e.time_range.start - t0) / 1e3:10.3f} ms  {e.time_range.elapsed_us():9.1f} us  {e.name[:110]}\n")
     # eager pass: per-kernel CUDA events (roofline) and the launch count
     eng.on, eng.launches = True, 0
-    ms_eager = timed(step_resident, args.steps)
+    ms_eager, _ = timed(step_resident, args.steps)
     launches = eng.launches
     eng.on = False
     t_fwd = sum(e0.elapsed_time(e1) for e0, e1 in eng.ev["fwd"]) / max(1, len(eng.ev["fwd"]))
@@ -485,11 +515,10 @@ def run_ours(args, rank, local_rank, world):
 
     sampler = ClockSampler(visible_gpu_index(local_rank))
     sampler.start()
-    if gstep is not None:
-        ms_total = timed(gstep.replay, args.steps)
-    else:
-        ms_total = timed(step_resident, args.steps)
+    ms_total, outs = timed(gstep.replay if gstep is not None else step_resident, args.steps)
     clocks = sampler.finish()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outs, group, rank, world)
 
     feeder = None
     if gstep is not None:
@@ -529,7 +558,7 @@ def run_ours(args, rank, local_rank, world):
     e2e_fn = step_e2e_graph if gstep is not None else step_e2e
     for _ in range(2):
         e2e_fn()
-    ms_e2e = timed(e2e_fn, args.steps)
+    ms_e2e, _ = timed(e2e_fn, args.steps)
     if args.timeline_e2e:
         # kernel / copy timeline of four host-fed steps (CUPTI through torch.profiler), rank 0 writes it as text
         from torch.profiler import profile, ProfilerActivity
@@ -554,7 +583,7 @@ def run_ours(args, rank, local_rank, world):
         for fl in _xchg._Pool.free.values():     # a barrier that timed out would have left its mark here
             for x in fl:
                 x.check()
-    final_loss = float((gstep.out[0] if gstep is not None else step_resident()).detach())
+    final_loss = float((gstep.out[0] if gstep is not None else step_resident()[0]).detach())
     if not math.isfinite(final_loss):
         raise RuntimeError(f"bench: loss is not finite ({final_loss})")
     parity = None
@@ -656,10 +685,15 @@ def main():
     ap.add_argument("--timeline-e2e", dest="timeline_e2e", default=None,
                     help="write a kernel / copy timeline of four host-fed (e2e) steps to this file")
     ap.add_argument("--trace", action="store_true", help="print a per-phase device-time breakdown of the step to stderr")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", default=None, metavar="DIR",
+                    help="write what the last timed step returned (loss, d_a, d_b, d_logit_scale; a seeded row sample of "
+                         "large gradients) to DIR/<name>.npy as float32")
     ap.add_argument("--comm", default="auto", choices=["auto", "link", "nccl"],
                     help="multi-GPU exchange: this repository's kernels over NVLink peer memory (link; the default where "
                          "available) or the NCCL collectives it is measured against")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     if args.comm != "auto":
         os.environ["CLIPNCE_COMM"] = args.comm

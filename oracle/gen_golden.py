@@ -1,11 +1,11 @@
 """Pin the oracle against the reference itself and write tests/golden/*.npz.
 
-Run in the BUILD container only (needs /root/reference; the GPU box has no copy):
+Needs a checkout of the reference project (SrikarK-code/clip-dplm), named by CLIP_DPLM_REFERENCE:
 
-    python oracle/gen_golden.py
+    CLIP_DPLM_REFERENCE=<checkout> python oracle/gen_golden.py
 
 What it does
-  1. imports the reference's own modules from /root/reference
+  1. imports the reference's own modules from that checkout
        - old/clip.py           RNAProteinCLIPModule / DiffMapProteinCLIPModule   (forward tail :63-67, :100-104)
        - old/clip_opt.py       optimized_clip_loss                               (:130-151)
        - tong/utils/losses.py  contrastive_loss                                  (:4-19)
@@ -13,7 +13,9 @@ What it does
      (current/tf_clip_codes (1).ipynb cell 41, raw :13146-13165, repeats the notebook lines above for three pairs with one
       shared logit scale; it is NOT loaded -- its loss is three calls of the pinned pair form)
   2. asserts oracle/ref_step.py reproduces each of them EXACTLY (torch.equal) on seeded inputs,
-  3. stores inputs (bf16-rounded, as uint16 bit patterns) + reference outputs as small fixtures.
+  3. stores inputs (bf16-rounded, as uint16 bit patterns) + reference outputs as small fixtures; fixtures with more
+     than GRAD_FULL_MAX gradient entries per side keep a seeded sample of GRAD_SAMPLE_ROWS gradient rows (`grad_rows`),
+     so that every file stays under 1 MB.
 
 Nothing here is imported by the product path.
 """
@@ -33,11 +35,19 @@ import torch.nn.functional as F
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF = "/root/reference"
+REF = os.environ.get("CLIP_DPLM_REFERENCE", "")
 sys.path.insert(0, ROOT)
 from oracle import ref_step as O  # noqa: E402
 
 OUT = os.path.join(ROOT, "tests", "golden")
+GRAD_FULL_MAX, GRAD_SAMPLE_ROWS = 1 << 16, 64
+
+
+def grad_rows(n, d):
+    """Rows of d_a64 / d_b64 a fixture stores: all of them, or a fixed seeded sample for the larger fixtures."""
+    if n * d <= GRAD_FULL_MAX:
+        return None
+    return np.sort(np.random.default_rng(0).choice(n, size=GRAD_SAMPLE_ROWS, replace=False))
 
 
 def _load(path, name):
@@ -48,6 +58,8 @@ def _load(path, name):
 
 
 def load_reference():
+    if not os.path.isdir(REF):
+        sys.exit("gen_golden: set CLIP_DPLM_REFERENCE to a checkout of the reference project")
     ref = {}
     # old/clip.py imports `configuration_hybrid_clip` (needs transformers; its ctor is broken on
     # transformers 5.5 -> duck-typed config below) -- stub the module so the import succeeds.
@@ -174,6 +186,9 @@ def main():
                     meta=np.array(json.dumps({k: v for k, v in kw.items() if not torch.is_tensor(v)})))
         if extra is not None:
             arrs["extra_bits"] = bf16_bits(extra)
+        rows = grad_rows(n, d)
+        if rows is not None:
+            arrs.update(grad_rows=rows, d_a64=arrs["d_a64"][rows], d_b64=arrs["d_b64"][rows])
         np.savez_compressed(os.path.join(OUT, name + ".npz"), **arrs)
         report["golden/" + name] = f"loss={float(r64['loss']):.6f}"
 

@@ -51,7 +51,8 @@ def test_oracle_reproduces_golden(path):
     ls = float(z["logit_scale"])
     r64 = O.ref_step(a.double(), b.double(), ls, **{k: (v.double() if torch.is_tensor(v) else v) for k, v in kw.items()})
     assert abs(float(r64["loss"]) - float(z["loss64"])) <= 1e-12 * max(1.0, abs(float(z["loss64"])))
-    assert rel(r64["d_a"].float(), z["d_a64"]) < 1e-6 and rel(r64["d_b"].float(), z["d_b64"]) < 1e-6
+    rows = z["grad_rows"] if "grad_rows" in z else slice(None)     # larger fixtures store a sample of gradient rows
+    assert rel(r64["d_a"].float()[rows], z["d_a64"]) < 1e-6 and rel(r64["d_b"].float()[rows], z["d_b64"]) < 1e-6
     r32 = O.ref_step(a, b, ls, **kw)
     assert abs(float(r32["loss"]) - float(z["loss32"])) <= 2e-6 * max(1.0, abs(float(z["loss32"])))
 
@@ -295,7 +296,12 @@ def test_sharded_retrieval_gloo():
 
 
 # ------------------------------------------------------------------------------------------------ drop-in surface
-@pytest.mark.skipif(not os.path.exists("/root/reference/old/clip.py"), reason="reference checkout only exists in the build container")
+REFERENCE = os.environ.get("CLIP_DPLM_REFERENCE")
+REFERENCE_CLIP = os.path.join(REFERENCE, "old", "clip.py") if REFERENCE else ""
+
+
+@pytest.mark.skipif(not os.path.isfile(REFERENCE_CLIP),
+                    reason="needs a checkout of the reference project named by CLIP_DPLM_REFERENCE")
 def test_module_parameter_names_match_reference():
     """state_dicts of the reference modules must load into the drop-in modules (same names and shapes)."""
     import importlib.util
@@ -304,7 +310,7 @@ def test_module_parameter_names_match_reference():
     stub = types.ModuleType("configuration_hybrid_clip")
     stub.HybridCLIPConfig = object
     sys.modules.setdefault("configuration_hybrid_clip", stub)
-    spec = importlib.util.spec_from_file_location("ref_old_clip_t", "/root/reference/old/clip.py")
+    spec = importlib.util.spec_from_file_location("ref_old_clip_t", REFERENCE_CLIP)
     ref = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(ref)
     from clip_dplm_b200 import modules as M
