@@ -63,7 +63,7 @@ SIGNATURES = {
     "clipnce_loss": [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _int, _vp, _vp],
     "clipnce_link_control_bytes": [ctypes.POINTER(_i64), ctypes.POINTER(_i64)],
     "clipnce_link_barrier": [ctypes.POINTER(_vp), _int, _int, _int, _vp],
-    "clipnce_link_push_rows": [_vp, _int, _i64, _i64, _int, ctypes.POINTER(_vp), _int, _int, _i64, _i64, _i64, _int, _vp],
+    "clipnce_link_push_rows": [_vp, _int, _i64, _i64, _int, ctypes.POINTER(_vp), _int, _int, _i64, _i64, _i64, _vp],
     "clipnce_link_copy": [_vp, _sz, ctypes.POINTER(_vp), _int, _int, _i64, _vp],
     "clipnce_link_epoch_advance": [ctypes.POINTER(_vp), _int, _int, _int, _vp],
     "clipnce_link_send_blocks": [_vp, _sz, _vp, _sz, ctypes.POINTER(_vp), _int, _int, _i64, _i64, _int, _vp],
@@ -130,7 +130,7 @@ def load():
             fn = getattr(lib, name)          # AttributeError here == header/library mismatch
             fn.argtypes = argtypes
             fn.restype = _RESTYPES.get(name, ctypes.c_int)
-        if lib.clipnce_version() != 108:
+        if lib.clipnce_version() != 109:
             raise RuntimeError("clip_dplm_b200: libclipnce.so version mismatch; rebuild")
         _lib = lib
         return lib

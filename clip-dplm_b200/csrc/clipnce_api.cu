@@ -10,7 +10,9 @@
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
+#include <set>
 #include <string>
+#include <utility>
 
 #include "../../include/clipnce.h"
 #include "kernels_aux.cuh"
@@ -41,11 +43,17 @@ int fail(int code, const char* fmt, ...) {
     if (e_ != cudaSuccess) return fail(CLIPNCE_ECUDA, "%s: %s", #expr, cudaGetErrorString(e_));     \
   } while (0)
 
+// Integer value of the environment variable `name`, `dflt` where it is unset.  Every CLIPNCE_* variable the library reads
+// goes through here (the list: INTEGRATION.md).  Test hooks are read on every call: tests switch them inside one process.
+long long env_int(const char* name, long long dflt) {
+  const char* e = getenv(name);
+  return e ? atoll(e) : dflt;
+}
+
 // a peer that does not arrive within this time is fatal (barriers and per-block waits trap)
 unsigned long long link_timeout_ns() {
   static const unsigned long long ns = [] {
-    const char* e = getenv("CLIPNCE_LINK_TIMEOUT_MS");
-    const long long ms = e ? atoll(e) : 600000;   // 10 minutes, the order of NCCL's watchdog; a timeout is fatal (trap)
+    const long long ms = env_int("CLIPNCE_LINK_TIMEOUT_MS", 600000);   // 10 minutes, the order of NCCL's watchdog
     return (unsigned long long)(ms > 0 ? ms : 600000) * 1000000ull;
   }();
   return ns;
@@ -56,11 +64,8 @@ inline int64_t round_up(int64_t a, int64_t b) { return ceil_div(a, b) * b; }
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 inline size_t elem_size(int dtype) { return dtype == CLIPNCE_BF16 ? 2 : 4; }
 
-// CTA-pair kernels (kernels_pair.cuh): the main tensor-core path.  CLIPNCE_NO_PAIR=1 forces the single-CTA kernels.
-bool pair_eligible(int64_t d) {
-  static const bool off = [] { const char* e = getenv("CLIPNCE_NO_PAIR"); return e && atoi(e) != 0; }();
-  return !off && d % 128 == 0 && d >= 128 && d <= 768;
-}
+// CTA-pair kernels (kernels_pair.cuh): the main tensor-core path.
+bool pair_eligible(int64_t d) { return d % 128 == 0 && d >= 128 && d <= 768; }
 
 // Kernel family.  0: exact CUDA-core kernels (fp32 check mode, shapes the tensor-core kernels do not take).
 // 1: tensor cores with the FIXED shift -- |S_ij| <= s, so exp(S - s) needs no running maximum; valid while e^(-2s) is a
@@ -81,7 +86,7 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 std::mutex g_mu;
 EncodeTiledFn g_encode = nullptr;
-bool g_attr_done[32] = {};
+std::set<std::pair<const void*, int>> g_smem_allowed;   // (kernel, device) pairs whose shared-memory limit is raised
 
 int get_encode(EncodeTiledFn* out) {
   std::lock_guard<std::mutex> lk(g_mu);
@@ -115,6 +120,20 @@ int make_tmap(CUtensorMap* m, const void* base, int64_t inner, int64_t outer, in
   return 0;
 }
 
+// Let `kern` take `bytes` of dynamic shared memory.  The attribute belongs to the kernel as loaded on one device, so it
+// is set once per (kernel, current device).
+template <typename Kernel>
+int allow_smem(Kernel* kern, int bytes) {
+  int dev = 0;
+  CUDA_TRY(cudaGetDevice(&dev));
+  const std::pair<const void*, int> key(reinterpret_cast<const void*>(kern), dev);
+  std::lock_guard<std::mutex> lk(g_mu);
+  if (g_smem_allowed.count(key)) return 0;
+  CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+  g_smem_allowed.insert(key);
+  return 0;
+}
+
 int check_device_sm100() {
   int dev = 0;
   CUDA_TRY(cudaGetDevice(&dev));
@@ -125,7 +144,7 @@ int check_device_sm100() {
 }
 
 template <int MODE, int BLOCK_I>
-int launch_tc(int attr_slot, const CUtensorMap& tx, const CUtensorMap& ty, const CUtensorMap& tyt, tc::Params p,
+int launch_tc(const CUtensorMap& tx, const CUtensorMap& ty, const CUtensorMap& tyt, tc::Params p,
               int grid, cudaStream_t st) {
   auto kern = tc::clip_tc_kernel<MODE, BLOCK_I>;
   const int fixed = tc::smem_bytes(MODE, BLOCK_I, p.nkc, 0);
@@ -140,13 +159,7 @@ int launch_tc(int attr_slot, const CUtensorMap& tx, const CUtensorMap& ty, const
     p.stages_b = 0;
   }
   const int smem = tc::smem_bytes(MODE, BLOCK_I, p.nkc, p.stages_a + p.stages_b);
-  {
-    std::lock_guard<std::mutex> lk(g_mu);
-    if (!g_attr_done[attr_slot]) {
-      CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_LIMIT));
-      g_attr_done[attr_slot] = true;
-    }
-  }
+  if (int rc = allow_smem(kern, tc::SMEM_LIMIT)) return rc;
   kern<<<grid, tc::num_threads(MODE, BLOCK_I), smem, st>>>(tx, ty, tyt, p);
   CUDA_TRY(cudaGetLastError());
   return 0;
@@ -164,8 +177,8 @@ int pair_slots() {   // CTA pairs that can be resident at once: one per two SMs
 // Cut a row block's column sweep into work items so that the grid fills whole waves of CTA pairs; every item pays a
 // fixed prologue / drain (~0.75 step), so fewer, longer items win ties.  Returns steps per item.
 int pick_split_steps(int n_pairs, int n_steps, int max_split) {
-  if (const char* e = getenv("CLIPNCE_SPLIT_STEPS")) {   // test hook: force the number of steps per work item
-    const int v = atoi(e);
+  {   // test hook: force the number of steps per work item
+    const int v = (int)env_int("CLIPNCE_SPLIT_STEPS", 0);
     if (v >= 1) return (int)ceil_div(n_steps, v) <= max_split ? v : (int)ceil_div(n_steps, max_split);
   }
   const int slots = pair_slots();
@@ -182,7 +195,7 @@ int pick_split_steps(int n_pairs, int n_steps, int max_split) {
 }
 
 template <int ROWS, int MODE = 0, int KT = 1>
-int launch_pair_fwd(int attr_slot, const void* x, const void* y, pair::FwdParams p, cudaStream_t st) {
+int launch_pair_fwd(const void* x, const void* y, pair::FwdParams p, cudaStream_t st) {
   auto kern = pair::fwd_kernel<ROWS, MODE, KT>;
   int stages = (pair::SMEM_LIMIT - pair::fwd_smem_bytes(ROWS, p.nkc, 0)) / pair::STAGE_BYTES;
   if (stages > pair::MAX_STAGES) stages = pair::MAX_STAGES;
@@ -193,26 +206,11 @@ int launch_pair_fwd(int attr_slot, const void* x, const void* y, pair::FwdParams
   // several problems in one launch: both operands are members of one stacked matrix, indexed by stack row
   if ((rc = make_tmap(&tx, x, p.d, p.grp.n_prob ? p.grp.stack_rows : p.n_rows, p.d, ROWS))) return rc;
   if ((rc = make_tmap(&ty, y, p.d, p.grp.n_prob ? p.grp.stack_rows : p.n_cols, p.d, 128))) return rc;
-  {
-    std::lock_guard<std::mutex> lk(g_mu);
-    if (!g_attr_done[attr_slot]) {
-      CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, pair::SMEM_LIMIT));
-      g_attr_done[attr_slot] = true;
-    }
-  }
+  if ((rc = allow_smem(kern, pair::SMEM_LIMIT))) return rc;
   const int grid = 2 * p.n_pairs * (int)ceil_div(p.n_steps, p.split_steps);
   kern<<<grid, pair::FWD_THREADS, pair::fwd_smem_bytes(ROWS, p.nkc, stages), st>>>(tx, ty, p);
   CUDA_TRY(cudaGetLastError());
   return 0;
-}
-
-// 4-CTA clusters with the streamed tiles multicast to both pairs (pair::bwd_body<.., MC>).  Measured on a B200 at
-// N = 65536, d = 512 (tools/run_mc_ab.sh, parity green both ways): 7.43 ms per side against 7.04 ms with 2-CTA clusters --
-// the sweep is bound per SM (shared-memory port), not by L2 output, and 4-CTA clusters leave SMs of the 18-SM GPCs idle.
-// Off unless CLIPNCE_BWD_MC=1.
-bool bwd_mc_enabled() {
-  static const bool on = [] { const char* e = getenv("CLIPNCE_BWD_MC"); return e && atoi(e) != 0; }();
-  return on;
 }
 
 template <bool TWO_EXP>
@@ -230,44 +228,15 @@ int launch_pair_bwd(const void* x, const void* y, pair::BwdParams p, cudaStream_
   if ((rc = make_tmap(&ty, y, p.d, y_rows, p.d, 128))) return rc;
   if ((rc = make_tmap(&tyg, y, p.d, y_rows, p.d, 64))) return rc;
   const size_t smem = pair::bwd_smem_bytes(p.nkc, p.stages_a + p.stages_b);
-  // two pairs per cluster share every streamed tile: needs an even number of row blocks (and, grouped, per problem)
-  const bool mc = bwd_mc_enabled() && p.n_pairs % 2 == 0 && (p.grp.n_prob == 0 || p.grp.pairs_per_prob % 2 == 0);
   const int grid = 2 * p.n_pairs * (int)ceil_div(p.n_steps, p.split_steps);
-  if (mc) {
-    auto kern = pair::bwd_kernel_mc<TWO_EXP>;
-    constexpr int attr_slot = TWO_EXP ? 21 : 20;
-    {
-      std::lock_guard<std::mutex> lk(g_mu);
-      if (!g_attr_done[attr_slot]) {
-        CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, pair::SMEM_LIMIT));
-        g_attr_done[attr_slot] = true;
-      }
-    }
-    kern<<<grid, pair::BWD_THREADS, smem, st>>>(tx, ty, tyg, p);
-  } else {
-    auto kern = pair::bwd_kernel<TWO_EXP>;
-    constexpr int attr_slot = TWO_EXP ? 12 : 6;
-    {
-      std::lock_guard<std::mutex> lk(g_mu);
-      if (!g_attr_done[attr_slot]) {
-        CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, pair::SMEM_LIMIT));
-        g_attr_done[attr_slot] = true;
-      }
-    }
-    kern<<<grid, pair::BWD_THREADS, smem, st>>>(tx, ty, tyg, p);
-  }
+  auto kern = pair::bwd_kernel<TWO_EXP>;
+  if ((rc = allow_smem(kern, pair::SMEM_LIMIT))) return rc;
+  kern<<<grid, pair::BWD_THREADS, smem, st>>>(tx, ty, tyg, p);
   CUDA_TRY(cudaGetLastError());
   return 0;
 }
 
 int fwd_block_i(int64_t n_rows, int64_t d) { return (d <= 512 && n_rows >= 128 * 148) ? 128 : 64; }
-// 64 rows (two logits buffers, deeper rings) measured faster than 96 rows (one buffer, 16 KiB stages) on B200
-// (9.6 vs 11.4 ms per side at N = 65536, d = 512); CLIPNCE_BWD_ROWS=96 selects the wider variant.
-int bwd_block_i(int64_t d) {
-  const char* e = getenv("CLIPNCE_BWD_ROWS");
-  if (e && atoi(e) == 96 && d <= 512) return 96;
-  return 64;
-}
 
 struct SimtFwdWs {
   float *row_pm, *row_pl, *col_pm, *col_pl;
@@ -429,7 +398,7 @@ int forward_impl(const void* x, const void* y, const float* rinv_x, const float*
     // (any scale: beyond ~105 more rows fall under the bound and the fallback runs more often, the results stay exact;
     // the decision must not depend on the scale -- ranks of a row-sharded step hold slightly different host copies of it)
     const bool speculate = !(flags & CLIPNCE_FLAG_UNBOUNDED) && n_cols <= (1ll << 22) && n_rows <= (1ll << 22) &&
-                           !getenv("CLIPNCE_NO_SPECULATE");
+                           env_int("CLIPNCE_NO_SPECULATE", 0) == 0;
     if (gat && !speculate) return fail(CLIPNCE_EUNSUPPORTED, "forward_gathered: no fixed-shift sweep for these arguments");
     if (speculate) {
       constexpr float kOff = 72.f;
@@ -454,7 +423,7 @@ int forward_impl(const void* x, const void* y, const float* rinv_x, const float*
       int* flag = reinterpret_cast<int*>(reinterpret_cast<char*>(workspace) + need - 256);
       CUDA_TRY(cudaMemsetAsync(flag, 0, sizeof(int), st));
       set_gathered(p, gat);
-      rc = rows == 128 ? launch_pair_fwd<128>(4, x, y, p, st) : launch_pair_fwd<64>(5, x, y, p, st);
+      rc = rows == 128 ? launch_pair_fwd<128>(x, y, p, st) : launch_pair_fwd<64>(x, y, p, st);
       if (rc) return rc;
       aux::reduce_shifted_partials<<<(unsigned)ceil_div(n_cols, 256), 256, 0, st>>>(p.col_part, n_part, p.col_ld, n_cols, scale,
                                                                                       scale_dev, kOff, thr_col, col_m, col_l, flag);
@@ -485,7 +454,7 @@ int forward_impl(const void* x, const void* y, const float* rinv_x, const float*
       used = need;
       const void* xs = side == 0 ? x : y;
       const void* ys = side == 0 ? y : x;
-      rc = rows == 128 ? launch_pair_fwd<128, 2>(7, xs, ys, p, st) : launch_pair_fwd<64, 2>(11, xs, ys, p, st);
+      rc = rows == 128 ? launch_pair_fwd<128, 2>(xs, ys, p, st) : launch_pair_fwd<64, 2>(xs, ys, p, st);
       if (rc) return rc;
       aux::reduce_ml_partials<<<(unsigned)ceil_div(nr, 256), 256, 0, st>>>(p.row_part_m, p.row_part, n_split, nr, nr,
                                                                             side == 0 ? row_m : col_m, side == 0 ? row_l : col_l, gate);
@@ -515,7 +484,7 @@ int forward_impl(const void* x, const void* y, const float* rinv_x, const float*
       p.col_part = reinterpret_cast<float*>(workspace);
       p.row_part = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + col_bytes);
       set_gathered(p, gat);
-      rc = rows == 128 ? launch_pair_fwd<128>(4, x, y, p, st) : launch_pair_fwd<64>(5, x, y, p, st);
+      rc = rows == 128 ? launch_pair_fwd<128>(x, y, p, st) : launch_pair_fwd<64>(x, y, p, st);
       if (rc) return rc;
       aux::reduce_col_partials<<<(unsigned)ceil_div(n_cols, 256), 256, 0, st>>>(p.col_part, n_part, p.col_ld, n_cols, scale,
                                                                                   scale_dev, col_m, col_l);
@@ -539,8 +508,8 @@ int forward_impl(const void* x, const void* y, const float* rinv_x, const float*
     p.diag_offset = diag_offset; p.scale = scale; p.k2 = scale * tc::LOG2E; p.scale_dev = scale_dev;
     p.rinv_x = rinv_x; p.rinv_y = rinv_y;
     p.row_m = row_m; p.row_l = row_l; p.col_part = reinterpret_cast<float*>(workspace); p.col_ld = col_ld; p.diag = diag;
-    if (bi == 128) rc = launch_tc<0, 128>(0, tx, ty, ty, p, (int)n_ib, st);
-    else           rc = launch_tc<0, 64>(1, tx, ty, ty, p, (int)n_ib, st);
+    if (bi == 128) rc = launch_tc<0, 128>(tx, ty, ty, p, (int)n_ib, st);
+    else           rc = launch_tc<0, 64>(tx, ty, ty, p, (int)n_ib, st);
     if (rc) return rc;
     aux::reduce_col_partials<<<(unsigned)ceil_div(n_cols, 256), 256, 0, st>>>(p.col_part, (int)((bi / 32) * n_ib), col_ld,
                                                                                 n_cols, scale, scale_dev, col_m, col_l);
@@ -584,7 +553,7 @@ int clipnce_forward(const void* x, const void* y, const float* rinv_x, const flo
 int clipnce_forward_gathered_ok(int dtype, int64_t d, float scale, int flags) {
   const int fam = tc_family(dtype, d, scale, flags);
   if (fam == 1) return pair_eligible(d) ? 1 : 0;
-  return (fam == 2 && !(flags & CLIPNCE_FLAG_UNBOUNDED) && !getenv("CLIPNCE_NO_SPECULATE")) ? 1 : 0;
+  return (fam == 2 && !(flags & CLIPNCE_FLAG_UNBOUNDED) && env_int("CLIPNCE_NO_SPECULATE", 0) == 0) ? 1 : 0;
 }
 
 int clipnce_forward_gathered(const void* x, const void* y, const float* rinv_x, const float* rinv_y, int64_t n_rows,
@@ -685,9 +654,9 @@ int backward_impl(const void* x, const void* y, const void* y_t, int64_t ld_t, c
     if (ld_t < n_cols || ld_t % 8 != 0) return fail(CLIPNCE_EINVAL, "backward: ld_t must be >= n_cols and a multiple of 8");
     if (!aligned16(x) || !aligned16(y) || !aligned16(y_t))
       return fail(CLIPNCE_EINVAL, "backward: operands must be 16-byte aligned");
-    // rows per CTA: the gradient accumulators (ceil(d/128) * BLOCK_I TMEM columns) plus the logits buffer(s) share
-    // the 512 TMEM columns -> 96 rows with one logits buffer up to d = 512, else 64 rows with two
-    const int bi = bwd_block_i(d);
+    // rows per CTA: the gradient accumulators (ceil(d/128) * BLOCK_I TMEM columns) plus two logits buffers share the
+    // 512 TMEM columns (measured on a B200 at N = 65536, d = 512: 9.6 ms per side, against 11.4 with 96 rows and one buffer)
+    const int bi = 64;
     const int64_t n_ib = ceil_div(n_rows, bi);
     const size_t need = sizeof(float) * (size_t)n_ib;
     if (workspace_bytes < need) return fail(CLIPNCE_EWORKSPACE, "backward: workspace %zu < %zu", workspace_bytes, need);
@@ -703,9 +672,7 @@ int backward_impl(const void* x, const void* y, const void* y_t, int64_t ld_t, c
     p.rinv_x = rinv_x; p.rinv_y = rinv_y;
     p.row_m_in = row_m; p.row_w = row_w; p.col_m_in = col_m; p.col_w = col_w; p.diag_w = diag_w; p.out_scale = grad_out * scale;
     p.dx = dx_hat; p.ds_part = d_scale_sum ? reinterpret_cast<float*>(workspace) : nullptr;
-    if (bi == 96) rc = launch_tc<1, 96>(3, tx, ty, tyt, p, (int)n_ib, st);
-    else          rc = launch_tc<1, 64>(2, tx, ty, tyt, p, (int)n_ib, st);
-    if (rc) return rc;
+    if ((rc = launch_tc<1, 64>(tx, ty, tyt, p, (int)n_ib, st))) return rc;
     if (d_scale_sum) {
       aux::reduce_scalar_partials<<<1, 32, 0, st>>>(p.ds_part, (int)n_ib, grad_out, d_scale_sum);
       CUDA_TRY(cudaGetLastError());
@@ -923,7 +890,7 @@ int clipnce_group_forward(const void* stack, const float* rinv, int n_members, i
 
   const int* gate = nullptr;
   size_t exact_off = 0;   // floats: where the exact sweeps' partials start
-  if (pl.fam == 2 && !getenv("CLIPNCE_NO_SPECULATE")) {
+  if (pl.fam == 2 && env_int("CLIPNCE_NO_SPECULATE", 0) == 0) {
     // bounded logits: one fixed-shift sweep with the shift lowered to s - 72, the exact sweeps gated on a device flag
     // (see clipnce_forward)
     constexpr float kOff = 72.f;
@@ -941,7 +908,7 @@ int clipnce_group_forward(const void* stack, const float* rinv, int n_members, i
     exact_off = (size_t)round_up((int64_t)(((size_t)n_part + (size_t)n_split) * (size_t)V), 64) + 64;
     int* flag = reinterpret_cast<int*>(wsf + exact_off - 64);
     CUDA_TRY(cudaMemsetAsync(flag, 0, sizeof(int), st));
-    rc = pl.rows == 128 ? launch_pair_fwd<128>(4, stack, stack, p, st) : launch_pair_fwd<64>(5, stack, stack, p, st);
+    rc = pl.rows == 128 ? launch_pair_fwd<128>(stack, stack, p, st) : launch_pair_fwd<64>(stack, stack, p, st);
     if (rc) return rc;
     aux::reduce_shifted_partials<<<(unsigned)ceil_div(V, 256), 256, 0, st>>>(p.col_part, n_part, V, V, scale, scale_dev, kOff, thr,
                                                                               stat_m + V, stat_l + V, flag, pl.n_pad, n);
@@ -962,7 +929,7 @@ int clipnce_group_forward(const void* stack, const float* rinv, int n_members, i
       p.diag = side == 0 ? diag : nullptr;
       p.row_part_m = wsf + exact_off + (size_t)side * 2 * (size_t)n_split * (size_t)V;
       p.row_part = p.row_part_m + (size_t)n_split * (size_t)V;
-      rc = pl.rows == 128 ? launch_pair_fwd<128, 2>(7, stack, stack, p, st) : launch_pair_fwd<64, 2>(11, stack, stack, p, st);
+      rc = pl.rows == 128 ? launch_pair_fwd<128, 2>(stack, stack, p, st) : launch_pair_fwd<64, 2>(stack, stack, p, st);
       if (rc) return rc;
       aux::reduce_ml_partials<<<(unsigned)ceil_div(V, 256), 256, 0, st>>>(p.row_part_m, p.row_part, n_split, V, V,
                                                                            stat_m + side * V, stat_l + side * V, gate);
@@ -978,7 +945,7 @@ int clipnce_group_forward(const void* stack, const float* rinv, int n_members, i
     const int n_part = 2 * pl.fwd_pairs;
     p.col_part = wsf;
     p.row_part = wsf + (size_t)n_part * (size_t)V;
-    rc = pl.rows == 128 ? launch_pair_fwd<128>(4, stack, stack, p, st) : launch_pair_fwd<64>(5, stack, stack, p, st);
+    rc = pl.rows == 128 ? launch_pair_fwd<128>(stack, stack, p, st) : launch_pair_fwd<64>(stack, stack, p, st);
     if (rc) return rc;
     aux::reduce_col_partials<<<(unsigned)ceil_div(V, 256), 256, 0, st>>>(p.col_part, n_part, V, V, scale, scale_dev,
                                                                           stat_m + V, stat_l + V);
@@ -1078,21 +1045,18 @@ int clipnce_group_backward(const void* stack, const float* rinv, int n_members, 
 // ---- two-sided backward (kernels_pair2.cuh) ----------------------------------------------------------------------------
 namespace {
 struct Bwd2Plan {
-  int P, Q, n_rb, n_seg, seg_steps, n_items, n_rounds, n_steps, n_half, depth, stages_a, stages_b, stages_c, gbuf, smem;
+  int P, Q, n_rb, n_seg, seg_steps, n_items, n_rounds, n_steps, n_half, depth, stages_a, stages_b, stages_c, smem;
   size_t off_flags, off_ring, off_dxh, off_dyh, off_part, bytes;
 };
 
 bool bwd2_device_ok() {   // every CTA pair of the persistent grid must be resident at once
-  {   // read per call: tests switch between the two-sided kernel and the two-sweep path inside one process
-    const char* e = getenv("CLIPNCE_NO_BWD2");
-    if (e && atoi(e) != 0) return false;
+  if (env_int("CLIPNCE_NO_BWD2", 0) != 0) return false;   // test hook: the two-sweep path instead
+  // the occupancy query below counts on the raised shared-memory limit
+  if (allow_smem(pair2::bwd2_kernel<false>, pair::SMEM_LIMIT) || allow_smem(pair2::bwd2_kernel<true>, pair::SMEM_LIMIT)) {
+    cudaGetLastError();
+    return false;
   }
   static const bool ok = [] {
-    if (cudaFuncSetAttribute(pair2::bwd2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, pair::SMEM_LIMIT) != cudaSuccess ||
-        cudaFuncSetAttribute(pair2::bwd2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, pair::SMEM_LIMIT) != cudaSuccess) {
-      cudaGetLastError();
-      return false;
-    }
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof cfg);
     cfg.gridDim = dim3(2 * pair_slots());
@@ -1120,9 +1084,8 @@ bool bwd2_plan(int64_t n_rows, int64_t n_cols, int64_t d, int dtype, float scale
   if (world == 0 ? n_rows != n_cols : n_rows * world != n_cols) return false;
   // below this the items do not fill the producer pairs; measured on one GPU, d = 512 (tools/run_bwd2_threshold.sh): 12288 rows
   // 0.571 ms per step against 0.692 with two sweeps, 8192 rows 0.329 against 0.307 (CLIPNCE_BWD2_MIN_N: test hook)
-  int64_t min_pairs = 12288ll * 12288ll;
-  if (const char* e = getenv("CLIPNCE_BWD2_MIN_N")) min_pairs = atoll(e) * atoll(e);
-  if (n_rows % 128 != 0 || n_cols % 256 != 0 || n_rows * n_cols < min_pairs || n_cols > (1ll << 22)) return false;
+  const int64_t min_n = env_int("CLIPNCE_BWD2_MIN_N", 12288);
+  if (n_rows % 128 != 0 || n_cols % 256 != 0 || n_rows * n_cols < min_n * min_n || n_cols > (1ll << 22)) return false;
   if (world >= 2 && (n_cols / world) % 256 != 0) return false;
   const int slots = pair_slots();
   if (slots < 8) return false;
@@ -1133,12 +1096,10 @@ bool bwd2_plan(int64_t n_rows, int64_t n_cols, int64_t d, int dtype, float scale
   // one producer step: a producer item costs seg_steps + 1 (accumulator drain, reload of the resident rows, pipeline
   // refill), the consumers work through one tile unit per producer tile at `r` times a producer's rate (measured on B200,
   // N = 65536, d = 512: P = 48..52 within 1 %), every segment beyond the first costs a pass over an [n_rows, d] fp32 slab.
-  const char* ef = getenv("CLIPNCE_BWD2_P");
-  const int forced_p = ef ? atoi(ef) : 0;
-  const char* es = getenv("CLIPNCE_BWD2_SEG");
-  const int forced_seg = es ? atoi(es) : 0;
-  const char* er = getenv("CLIPNCE_BWD2_RATIO");
-  const double r = (er && atof(er) > 0.1) ? atof(er) : 1.0;
+  // CLIPNCE_BWD2_P / CLIPNCE_BWD2_SEG (test hooks) force the split and the number of segments.
+  const int forced_p = (int)env_int("CLIPNCE_BWD2_P", 0);
+  const int forced_seg = (int)env_int("CLIPNCE_BWD2_SEG", 0);
+  constexpr double r = 1.0;
   double best_t = 1e300;
   int best_p = 0, best_seg = 0;
   for (int n_seg = 1; n_seg <= 8; n_seg *= 2) {
@@ -1169,18 +1130,14 @@ bool bwd2_plan(int64_t n_rows, int64_t n_cols, int64_t d, int dtype, float scale
   pl->n_items = pl->n_rb * best_seg;
   pl->n_rounds = (int)ceil_div(pl->n_items, pl->P);
   pl->depth = pair2::RING_DEPTH;
-  if (const char* e = getenv("CLIPNCE_BWD2_DEPTH")) { const int v = atoi(e); if (v >= 2 && v <= 64) pl->depth = v; }
   const int nkc = (int)(d / 64);
-  pl->gbuf = 1;
-  if (const char* e = getenv("CLIPNCE_BWD2_GBUF")) { if (atoi(e) == 2) pl->gbuf = 2; }
-  int total = (pair::SMEM_LIMIT - pair2::producer_smem(nkc, 0, pl->gbuf)) / pair::STAGE_BYTES;
-  if (total < 4 && pl->gbuf == 2) { pl->gbuf = 1; total = (pair::SMEM_LIMIT - pair2::producer_smem(nkc, 0, 1)) / pair::STAGE_BYTES; }
+  const int total = (pair::SMEM_LIMIT - pair2::producer_smem(nkc, 0)) / pair::STAGE_BYTES;
   if (total < 4) return false;
   auto cap = [](int v) { return v > pair2::MAXS ? pair2::MAXS : v; };
   pl->stages_b = cap(total / 2);
   pl->stages_a = cap(total - total / 2);
   pl->stages_c = cap((pair::SMEM_LIMIT - pair2::consumer_smem(0)) / pair2::C_STAGE);
-  const int ps = pair2::producer_smem(nkc, pl->stages_a + pl->stages_b, pl->gbuf), cs = pair2::consumer_smem(pl->stages_c);
+  const int ps = pair2::producer_smem(nkc, pl->stages_a + pl->stages_b), cs = pair2::consumer_smem(pl->stages_c);
   pl->smem = ps > cs ? ps : cs;
   size_t off = 0;
   auto region = [&](size_t bytes) { const size_t o = off; off = (size_t)round_up((int64_t)(off + bytes), 256); return o; };
@@ -1226,11 +1183,7 @@ int bwd2_launch(const Bwd2Plan& pl, const void* x, const void* y, const float* r
   p.nsbuf = p.nq2 <= 2 ? 2 : 1;   // 128 nq2 accumulator columns + 128 per logits buffer <= 512
   p.n_rb = pl.n_rb; p.n_seg = pl.n_seg; p.seg_steps = pl.seg_steps; p.n_items = pl.n_items; p.n_rounds = pl.n_rounds;
   p.P = pl.P; p.Q = pl.Q; p.depth = pl.depth;
-  p.stages_a = pl.stages_a; p.stages_b = pl.stages_b; p.stages_c = pl.stages_c; p.gbuf = pl.gbuf;
-  {
-    const char* e = getenv("CLIPNCE_BWD2_L2HINT");
-    p.l2_hints = e ? atoi(e) : 1;
-  }
+  p.stages_a = pl.stages_a; p.stages_b = pl.stages_b; p.stages_c = pl.stages_c;
   p.diag_offset = diag_offset; p.scale = scale; p.scale_dev = scale_dev; p.diag_w = diag_w;
   p.rinv_x = rinv_x; p.rinv_y = rinv_y; p.row_m = row_m; p.row_w = row_w; p.col_m = col_m; p.col_w = col_w;
   p.dx = reinterpret_cast<float*>(ws + pl.off_dxh);
@@ -1244,10 +1197,9 @@ int bwd2_launch(const Bwd2Plan& pl, const void* x, const void* y, const float* r
   if ((rc = make_tmap(&ty, y, d, n_cols, d, 128))) return rc;
   if ((rc = make_tmap(&tyg, y, d, n_cols, d, 64))) return rc;
   if ((rc = make_tmap(&tg, ws + pl.off_ring, 256, (int64_t)pl.depth * pl.P * 128, 256, 64))) return rc;
-  if (tc_family(CLIPNCE_BF16, d, scale, 0) == 2)
-    pair2::bwd2_kernel<true><<<2 * (pl.P + pl.Q), pair2::THREADS, pl.smem, st>>>(tx, ty, tyg, tg, p);
-  else
-    pair2::bwd2_kernel<false><<<2 * (pl.P + pl.Q), pair2::THREADS, pl.smem, st>>>(tx, ty, tyg, tg, p);
+  auto kern = tc_family(CLIPNCE_BF16, d, scale, 0) == 2 ? pair2::bwd2_kernel<true> : pair2::bwd2_kernel<false>;
+  if ((rc = allow_smem(kern, pair::SMEM_LIMIT))) return rc;
+  kern<<<2 * (pl.P + pl.Q), pair2::THREADS, pl.smem, st>>>(tx, ty, tyg, tg, p);
   CUDA_TRY(cudaGetLastError());
   return 0;
 }
@@ -1452,9 +1404,9 @@ int clipnce_topk(const void* q, const void* lib, const float* rinv_q, const floa
   p.cand_idx = reinterpret_cast<int*>(p.cand_score + pl.cand_elems);
   p.row_thr = p.cand_idx + pl.cand_elems;
   CUDA_TRY(cudaMemsetAsync(p.row_thr, 0x80, sizeof(int) * (size_t)n_q, st));   // key 0x80808080: below every real score
-  if (pl.kt == 1) rc = launch_pair_fwd<128, 1, 1>(8, q, lib, p, st);
-  else if (pl.kt == 10) rc = launch_pair_fwd<128, 1, 10>(9, q, lib, p, st);
-  else rc = launch_pair_fwd<128, 1, 16>(10, q, lib, p, st);
+  if (pl.kt == 1) rc = launch_pair_fwd<128, 1, 1>(q, lib, p, st);
+  else if (pl.kt == 10) rc = launch_pair_fwd<128, 1, 10>(q, lib, p, st);
+  else rc = launch_pair_fwd<128, 1, 16>(q, lib, p, st);
   if (rc) return rc;
   aux::topk_merge<<<(unsigned)ceil_div(n_q, 8), 256, 0, st>>>(p.cand_score, p.cand_idx, pl.n_split * 4, n_q, pl.kt, k, out_score,
                                                                out_idx);
@@ -1532,13 +1484,7 @@ int clipnce_head_tail(const void* h, const void* w, const float* bias, const flo
   CUtensorMap th, tw;
   if ((rc = make_tmap(&th, h, k, n, k, head::ROWS))) return rc;
   if ((rc = make_tmap(&tw, w, k, p, k, 128))) return rc;
-  {
-    std::lock_guard<std::mutex> lk(g_mu);
-    if (!g_attr_done[13]) {
-      CUDA_TRY(cudaFuncSetAttribute(head::linear_ln_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, pair::SMEM_LIMIT));
-      g_attr_done[13] = true;
-    }
-  }
+  if ((rc = allow_smem(head::linear_ln_kernel, pair::SMEM_LIMIT))) return rc;
   head::linear_ln_kernel<<<(unsigned)ceil_div(n, head::ROWS), head::THREADS, head::smem_bytes((int)p, stages), as_stream(stream)>>>(th, tw, hp);
   CUDA_TRY(cudaGetLastError());
   return 0;
@@ -1592,8 +1538,7 @@ int clipnce_link_barrier(void* const* peer_base, int world, int rank, int phase,
 }
 
 int clipnce_link_push_rows(const void* x, int in_dtype, int64_t n, int64_t d, int c_dtype, void* const* peer_base,
-                           int world, int rank, int64_t rows_offset, int64_t rinv_offset, int64_t row0, int max_blocks,
-                           void* stream) {
+                           int world, int rank, int64_t rows_offset, int64_t rinv_offset, int64_t row0, void* stream) {
   link::Peers peers;
   int rc = make_peers(peer_base, world, rank, &peers);
   if (rc) return rc;
@@ -1605,15 +1550,8 @@ int clipnce_link_push_rows(const void* x, int in_dtype, int64_t n, int64_t d, in
   if (in_dtype == CLIPNCE_BF16 && c_dtype == CLIPNCE_BF16 && (d % 8 != 0 || !aligned16(x)))
     return fail(CLIPNCE_EINVAL, "link_push_rows: bf16 rows need d %% 8 == 0 and 16-byte alignment");
   cudaStream_t st = as_stream(stream);
-  // foreground: one warp per row over the whole GPU.  Background (max_blocks > 0): a few fat grid-stride blocks
-  // (measured on 2 GPUs beside the forward sweep: 8 x 1024 threads cost it 1.60 ms -> small blocks 1.74 ms: blocks of
-  // another kernel are not placed next to a resident CTA pair, they take SMs as pairs retire, and many small blocks
-  // take many).  The step itself moves the A rows with the copy engines instead (clipnce_link_copy).
-  static const int bg_warps = [] { const char* e = getenv("CLIPNCE_LINK_BG_WARPS"); const int v = e ? atoi(e) : 32; return v >= 1 && v <= 32 ? v : 32; }();
-  const int wpb = max_blocks > 0 ? bg_warps : 8;
-  int64_t nblk = ceil_div(n, wpb);
-  if (max_blocks > 0 && nblk > max_blocks) nblk = max_blocks;
-  dim3 grid((unsigned)nblk), block(32 * wpb);
+  const int wpb = 8;   // one warp per row over the whole GPU
+  dim3 grid((unsigned)ceil_div(n, wpb)), block(32 * wpb);
   const int di = (int)d;
   if (in_dtype == CLIPNCE_BF16 && c_dtype == CLIPNCE_BF16)
     link::push_rows<__nv_bfloat16, __nv_bfloat16><<<grid, block, 0, st>>>((const __nv_bfloat16*)x, n, di, peers, world, rank, rows_offset, rinv_offset, row0);

@@ -137,24 +137,17 @@ __host__ __device__ constexpr int bwd_smem_bytes(int nkc, int stages) {
 // TWO_EXP = true: exp(S - m_i) w_i + exp(S - m_j) w_j with the (shift, sum) pairs as they are, two ex2 per logit: valid
 // for ANY logit range (s up to the clamp at 100, un-normalised queue rows), because every exponent is <= 0 by
 // construction of the shifts (true maxima, or s where |S| <= s).
-// MC = true: clusters of FOUR CTAs = two pairs working on adjacent row blocks of the same work-item column range.  Both pairs
-// stream the same Y tiles, so every box is fetched from L2 ONCE and multicast into the two CTAs that hold the same half
-// (ranks r and r + 2); the pairs take turns issuing.  The backward is bound by L2 -> SM bandwidth (every SM pulls 64 B/clk
-// of streamed operands for 128 resident rows per pair: 10-11 TB/s chip-wide, measured), which this halves.  A ring stage is
-// free when BOTH pairs' MMAs have read it: the EMPTY barriers count two commits, multicast to all four CTAs.
-template <bool TWO_EXP, bool MC>
-__device__ __forceinline__ void bwd_body(const CUtensorMap& tmap_x, const CUtensorMap& tmap_y, const CUtensorMap& tmap_yg,
-                                         const BwdParams& p) {
+template <bool TWO_EXP>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(BWD_THREADS, 1)
+bwd_kernel(const __grid_constant__ CUtensorMap tmap_x,    // X  box {64 k, 64 rows}
+           const __grid_constant__ CUtensorMap tmap_y,    // Y  box {64 k, 128 rows}   (logits operand, K-major)
+           const __grid_constant__ CUtensorMap tmap_yg,   // Y  box {64 d, 64 rows}    (gradient operand, MN-major)
+           const BwdParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const uint32_t base = ptx::smem_u32(smem);
   if ((base & 1023u) != 0) __trap();
-  const uint32_t crank = ptx::cluster_ctarank();
-  const uint32_t rank = crank & 1u;             // CTA within its pair
-  const uint32_t pr = MC ? (crank >> 1) : 0u;   // pair within the cluster
+  const uint32_t rank = ptx::cluster_ctarank() & 1u;   // CTA within its pair
   const bool leader = rank == 0;
-  const uint16_t pair_mask = static_cast<uint16_t>(3u << (2u * pr));       // commits that stay inside the pair
-  const uint16_t ring_mask = static_cast<uint16_t>(MC ? 0xFu : 0x3u);      // ring-stage releases: every CTA that issues TMA
-  const uint16_t mc_mask = static_cast<uint16_t>(5u << rank);              // the CTAs holding this CTA's half of a Y tile
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int item = blockIdx.x >> 1;
@@ -187,9 +180,9 @@ __device__ __forceinline__ void bwd_body(const CUtensorMap& tmap_x, const CUtens
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < MAX_STAGES; ++s) {
       ptx::mbar_init(bar(B_FULL_A + s), 1);
-      ptx::mbar_init(bar(B_EMPTY_A + s), MC ? 2 : 1);
+      ptx::mbar_init(bar(B_EMPTY_A + s), 1);
       ptx::mbar_init(bar(B_FULL_B + s), 1);
-      ptx::mbar_init(bar(B_EMPTY_B + s), MC ? 2 : 1);
+      ptx::mbar_init(bar(B_EMPTY_B + s), 1);
     }
     ptx::mbar_init(bar(B_XFULL), 1);
     for (int b = 0; b < 2; ++b) {
@@ -227,12 +220,8 @@ __device__ __forceinline__ void bwd_body(const CUtensorMap& tmap_x, const CUtens
         for (int g = 0; g < p.nkc; ++g) {
           ptx::mbar_wait(bar(B_EMPTY_A + stage), phase ^ 1u);
           if (leader) ptx::mbar_arrive_expect_tx(bar(B_FULL_A + stage), 2 * STAGE_BYTES);
-          if (!MC)
-            ptx::tma_load_2d_pair(ring_a + stage * STAGE_BYTES, &tmap_y, bar(B_FULL_A + stage), g * 64,
-                                  (t_begin + t) * STEP_J + (int)rank * 128 + gv.ys);
-          else if ((uint32_t)(g & 1) == pr)
-            ptx::tma_load_2d_pair_mc(ring_a + stage * STAGE_BYTES, &tmap_y, bar(B_FULL_A + stage), g * 64,
-                                     (t_begin + t) * STEP_J + (int)rank * 128 + gv.ys, mc_mask);
+          ptx::tma_load_2d_pair(ring_a + stage * STAGE_BYTES, &tmap_y, bar(B_FULL_A + stage), g * 64,
+                                (t_begin + t) * STEP_J + (int)rank * 128 + gv.ys);
           if (++stage == p.stages_a) { stage = 0; phase ^= 1u; }
         }
       }
@@ -251,15 +240,9 @@ __device__ __forceinline__ void bwd_body(const CUtensorMap& tmap_x, const CUtens
             const int ngr = half >> 6;                // 64-wide MN groups
             ptx::mbar_wait(bar(B_EMPTY_B + stage), phase ^ 1u);
             if (leader) ptx::mbar_arrive_expect_tx(bar(B_FULL_B + stage), 2 * ngr * 8192);
-            for (int gi = 0; gi < ngr; ++gi) {
-              if (!MC)
-                ptx::tma_load_2d_pair(ring_b + stage * STAGE_BYTES + gi * 8192, &tmap_yg, bar(B_FULL_B + stage),
-                                      256 * q + half * (int)rank + 64 * gi, (t_begin + t) * STEP_J + 64 * kc + gv.ys);
-              else if ((uint32_t)(kc & 1) == pr)
-                ptx::tma_load_2d_pair_mc(ring_b + stage * STAGE_BYTES + gi * 8192, &tmap_yg, bar(B_FULL_B + stage),
-                                         256 * q + half * (int)rank + 64 * gi, (t_begin + t) * STEP_J + 64 * kc + gv.ys,
-                                         mc_mask);
-            }
+            for (int gi = 0; gi < ngr; ++gi)
+              ptx::tma_load_2d_pair(ring_b + stage * STAGE_BYTES + gi * 8192, &tmap_yg, bar(B_FULL_B + stage),
+                                    256 * q + half * (int)rank + 64 * gi, (t_begin + t) * STEP_J + 64 * kc + gv.ys);
             if (++stage == p.stages_b) { stage = 0; phase ^= 1u; }
           }
         }
@@ -287,8 +270,8 @@ __device__ __forceinline__ void bwd_body(const CUtensorMap& tmap_x, const CUtens
           ready = ptx::mma_box_pair(d_tmem, mk(desc_hi_k, x_lo0 + g * (BWD_X_CHUNK >> 4)),
                                     mk(desc_hi_k, a_lo0 + stage * (STAGE_BYTES >> 4)), 2, 2, idesc_s, g != 0,
                                     bar(B_FULL_A + ns), np);
-          ptx::mma_commit_pair_mask(bar(B_EMPTY_A + stage), ring_mask);
-          if (g == p.nkc - 1) ptx::mma_commit_pair_mask(bar(B_SFULL + sb), pair_mask);
+          ptx::mma_commit_pair(bar(B_EMPTY_A + stage));
+          if (g == p.nkc - 1) ptx::mma_commit_pair(bar(B_SFULL + sb));
           stage = ns;
           phase = np;
         }
@@ -315,14 +298,14 @@ __device__ __forceinline__ void bwd_body(const CUtensorMap& tmap_x, const CUtens
             ready = ptx::mma_box_pair(tmem_base + 128 * q, mk(desc_hi_k, g_lo0 + kc * (8192 >> 4)),
                                       mk(desc_hi_mn, b_lo0 + stage * (STAGE_BYTES >> 4)), 2, 2048 >> 4, idesc_g,
                                       (t | kc) != 0, bar(B_FULL_B + ns), np);
-            ptx::mma_commit_pair_mask(bar(B_EMPTY_B + stage), ring_mask);
+            ptx::mma_commit_pair(bar(B_EMPTY_B + stage));
             stage = ns;
             phase = np;
           }
-          ptx::mma_commit_pair_mask(bar(B_GEMPTY + kc), pair_mask);
+          ptx::mma_commit_pair(bar(B_GEMPTY + kc));
         }
       }
-      ptx::mma_commit_pair_mask(bar(B_ACCFULL), pair_mask);
+      ptx::mma_commit_pair(bar(B_ACCFULL));
     }
     __syncwarp();
   } else {
@@ -345,8 +328,8 @@ __device__ __forceinline__ void bwd_body(const CUtensorMap& tmap_x, const CUtens
     const float rw = (TWO_EXP && row_ok) ? p.row_w[i_glob] : 0.f;
     const uint32_t g_row = g_smem + kc * 8192 + (i_local >> 3) * 1024 + (i_local & 7) * 128;
     const uint32_t sw = i_local & 7;
-    const uint32_t sempty_leader = ptx::mapa(bar(B_SEMPTY), 2u * pr);
-    const uint32_t gfull_leader = ptx::mapa(bar(B_GFULL + kc), 2u * pr);
+    const uint32_t sempty_leader = ptx::mapa(bar(B_SEMPTY), 0);
+    const uint32_t gfull_leader = ptx::mapa(bar(B_GFULL + kc), 0);
     const long long dcol0 = i_glob + p.diag_offset;   // column of this row's positive
 
     auto load_col = [&](int t, float& cw, float& cm, float& ry) {   // t: step local to this work item
@@ -465,21 +448,6 @@ __device__ __forceinline__ void bwd_body(const CUtensorMap& tmap_x, const CUtens
   __syncthreads();
   ptx::cluster_sync();   // the peer's shared memory / TMEM stay alive until every MMA of the pair has drained
   if (warp == 2) ptx::tmem_dealloc_pair(tmem_base, TMEM_COLS);
-}
-
-template <bool TWO_EXP>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(BWD_THREADS, 1)
-bwd_kernel(const __grid_constant__ CUtensorMap tmap_x,    // X  box {64 k, 64 rows}
-           const __grid_constant__ CUtensorMap tmap_y,    // Y  box {64 k, 128 rows}   (logits operand, K-major)
-           const __grid_constant__ CUtensorMap tmap_yg,   // Y  box {64 d, 64 rows}    (gradient operand, MN-major)
-           const BwdParams p) {
-  bwd_body<TWO_EXP, false>(tmap_x, tmap_y, tmap_yg, p);
-}
-template <bool TWO_EXP>
-__global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(BWD_THREADS, 1)
-bwd_kernel_mc(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__ CUtensorMap tmap_y,
-              const __grid_constant__ CUtensorMap tmap_yg, const BwdParams p) {
-  bwd_body<TWO_EXP, true>(tmap_x, tmap_y, tmap_yg, p);
 }
 
 // ===================================================================================================== forward

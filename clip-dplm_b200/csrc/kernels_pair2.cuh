@@ -65,8 +65,8 @@ constexpr int MAX_WORLD = 16;
 
 constexpr int B_FULL_A = 0, B_EMPTY_A = MAXS, B_FULL_B = 2 * MAXS, B_EMPTY_B = 3 * MAXS, B_XFULL = 4 * MAXS,
               B_XEMPTY = B_XFULL + 1, B_SFULL = B_XEMPTY + 1, B_SEMPTY = B_SFULL + 2, B_GFULL = B_SEMPTY + 2,
-              B_GEMPTY = B_GFULL + 8, B_ACCFULL = B_GEMPTY + 8, B_ACCEMPTY = B_ACCFULL + 2, B_GSFULL = B_ACCEMPTY + 2,
-              B_GSTORED = B_GSFULL + 8, B_COUNT = B_GSTORED + 8;      // G barriers: [buffer][box]
+              B_GEMPTY = B_GFULL + 4, B_ACCFULL = B_GEMPTY + 4, B_ACCEMPTY = B_ACCFULL + 2, B_GSFULL = B_ACCEMPTY + 2,
+              B_GSTORED = B_GSFULL + 4, B_COUNT = B_GSTORED + 4;      // G barriers: one per box
 static_assert(B_COUNT * 8 <= 1000, "barrier block");
 
 struct Params {
@@ -76,8 +76,6 @@ struct Params {
   int n_rb, n_seg, seg_steps, n_items, n_rounds;
   int P, Q, depth;
   int stages_a, stages_b, stages_c;
-  int gbuf;                   // 1 or 2 copies of the producer's G tile in shared memory
-  int l2_hints;               // ring stores / loads carry the evict_last L2 policy
   long long diag_offset;      // column of row i's positive = i + diag_offset
   float scale, diag_w;
   const float* scale_dev;
@@ -97,8 +95,8 @@ struct Params {
   uint32_t* done;             // [n_rounds * seg_steps]
 };
 
-__host__ __device__ constexpr int producer_smem(int nkc, int stages, int gbuf = 1) {
-  return nkc * X_CHUNK + gbuf * G_BYTES + stages * STAGE_BYTES + SMALL;
+__host__ __device__ constexpr int producer_smem(int nkc, int stages) {
+  return nkc * X_CHUNK + G_BYTES + stages * STAGE_BYTES + SMALL;
 }
 constexpr int FLUSH_BYTES = EPI_WARPS * 4096;   // consumer epilogue: one [32 rows][32 f32] transposing scratch per warp
 __host__ __device__ constexpr int consumer_smem(int stages) { return stages * C_STAGE + FLUSH_BYTES + SMALL; }
@@ -157,7 +155,7 @@ bwd2_kernel(const __grid_constant__ CUtensorMap tmap_x,    // X  box {64, 64 row
   const bool is_producer = pair_id < p.P;
 
   // the small block sits at the same offset for both roles: behind the larger of the two layouts
-  const int body = max(producer_smem(p.nkc, p.stages_a + p.stages_b, p.gbuf), consumer_smem(p.stages_c)) - SMALL;
+  const int body = max(producer_smem(p.nkc, p.stages_a + p.stages_b), consumer_smem(p.stages_c)) - SMALL;
   const uint32_t bars = base + body;
   auto bar = [&](int i) -> uint32_t { return bars + 8u * i; };
   volatile uint32_t* tmem_ptr_smem = reinterpret_cast<volatile uint32_t*>(smem + body + 1016);
@@ -187,7 +185,7 @@ bwd2_kernel(const __grid_constant__ CUtensorMap tmap_x,    // X  box {64, 64 row
       ptx::mbar_init(bar(B_ACCFULL + b), 1);
       ptx::mbar_init(bar(B_ACCEMPTY + b), 2 * EPI_WARPS);
     }
-    for (int k = 0; k < 8; ++k) {
+    for (int k = 0; k < 4; ++k) {
       ptx::mbar_init(bar(B_GFULL + k), 4);
       ptx::mbar_init(bar(B_GEMPTY + k), 1);
       ptx::mbar_init(bar(B_GSFULL + k), 2);     // the two epilogue warps of THIS CTA that wrote box k
@@ -212,11 +210,7 @@ bwd2_kernel(const __grid_constant__ CUtensorMap tmap_x,    // X  box {64, 64 row
     // item of round r: i = r P + pair_id  ->  segment i / n_rb, row block i % n_rb, column steps seg * seg_steps + tau
     const uint32_t x_smem = base;
     const uint32_t g_smem = x_smem + p.nkc * X_CHUNK;
-    const uint32_t ring_a = g_smem + p.gbuf * G_BYTES;
-    // G tile copy and barrier phase of global step counter gs: with two copies the epilogue writes step t while the dX
-    // MMAs and the ring store of step t-1 still read the other one
-    auto g_buf = [&](uint32_t gs) -> uint32_t { return p.gbuf == 2 ? (gs & 1u) : 0u; };
-    auto g_par = [&](uint32_t gs) -> uint32_t { return p.gbuf == 2 ? ((gs >> 1) & 1u) : (gs & 1u); };
+    const uint32_t ring_a = g_smem + G_BYTES;
     const uint32_t ring_b = ring_a + p.stages_a * STAGE_BYTES;
     const int S_COL0 = TMEM_COLS - 128 * p.nsbuf;   // logits buffers of 128 columns behind the accumulators
     auto s_buf = [&](uint32_t gs) -> int { return p.nsbuf == 2 ? (int)(gs & 1u) : 0; };
@@ -320,8 +314,7 @@ bwd2_kernel(const __grid_constant__ CUtensorMap tmap_x,    // X  box {64, 64 row
           ptx::tc_fence_after();
           for (int t = 0; t < p.seg_steps; ++t, ++gs) {
             for (int kc = 0; kc < 4; ++kc) {
-              const uint32_t gb = g_buf(gs);
-              ptx::mbar_wait(bar(B_GFULL + 4 * gb + kc), g_par(gs));
+              ptx::mbar_wait(bar(B_GFULL + kc), gs & 1u);
               for (int q = 0; q < p.nq2; ++q) {
                 const int wq = min(256, p.d - 256 * q);
                 const uint32_t idesc_g = ptx::idesc_bf16_f32_major(2 * ROWS, wq, 0, 1);
@@ -330,14 +323,14 @@ bwd2_kernel(const __grid_constant__ CUtensorMap tmap_x,    // X  box {64, 64 row
                 int ns = stage + 1;
                 uint32_t np = phase;
                 if (ns == p.stages_b) { ns = 0; np ^= 1u; }
-                ready = ptx::mma_box_pair(tmem_base + 128 * q, mk(desc_hi_k, g_lo0 + (gb * G_BYTES + kc * 8192 >> 4)),
+                ready = ptx::mma_box_pair(tmem_base + 128 * q, mk(desc_hi_k, g_lo0 + kc * (8192 >> 4)),
                                           mk(desc_hi_mn, b_lo0 + stage * (STAGE_BYTES >> 4)), 2, 2048 >> 4, idesc_g,
                                           (t | kc) != 0, bar(B_FULL_B + ns), np);
                 ptx::mma_commit_pair(bar(B_EMPTY_B + stage));
                 stage = ns;
                 phase = np;
               }
-              ptx::mma_commit_pair(bar(B_GEMPTY + 4 * gb + kc));
+              ptx::mma_commit_pair(bar(B_GEMPTY + kc));
             }
           }
           ptx::mma_commit_pair(bar(B_ACCFULL));
@@ -360,15 +353,13 @@ bwd2_kernel(const __grid_constant__ CUtensorMap tmap_x,    // X  box {64, 64 row
             const uint32_t g = (uint32_t)r * (uint32_t)p.seg_steps + (uint32_t)t;
             const int row0 = ((int)(g % (uint32_t)p.depth) * p.P + pair_id) * 128 + (int)rank * ROWS;
             // latency-critical part: the epilogue of the NEXT step waits for these boxes to be released
-            const uint32_t gb = g_buf(gs);
             for (int kc = 0; kc < 4; ++kc) {
-              ptx::mbar_wait(bar(B_GSFULL + 4 * gb + kc), g_par(gs));
-              if (p.l2_hints) ptx::tma_store_2d_hint(&tmap_g, g_smem + gb * G_BYTES + kc * 8192, 64 * kc, row0, keep);
-              else ptx::tma_store_2d(&tmap_g, g_smem + gb * G_BYTES + kc * 8192, 64 * kc, row0);
+              ptx::mbar_wait(bar(B_GSFULL + kc), gs & 1u);
+              ptx::tma_store_2d_hint(&tmap_g, g_smem + kc * 8192, 64 * kc, row0, keep);
               ptx::bulk_commit_group();
             }
             ptx::bulk_wait_group_read0();               // shared memory of the four boxes has been read
-            for (int kc = 0; kc < 4; ++kc) ptx::mbar_arrive(bar(B_GSTORED + 4 * gb + kc));
+            for (int kc = 0; kc < 4; ++kc) ptx::mbar_arrive(bar(B_GSTORED + kc));
             // off the critical path: publish the PREVIOUS step (its four groups are older than the four just committed,
             // so this does not wait for an L2 round trip), then the back-pressure check for the next step
             if (pending) {
@@ -400,10 +391,10 @@ bwd2_kernel(const __grid_constant__ CUtensorMap tmap_x,    // X  box {64, 64 row
       const int jl0 = 128 * jh + 64 * h;
       const int kc = 2 * jh + h;
       const uint32_t t_lane = tmem_base + (static_cast<uint32_t>(q * 32) << 16);
-      const uint32_t g_row0 = g_smem + kc * 8192 + (i_local >> 3) * 1024 + (i_local & 7) * 128;
+      const uint32_t g_row = g_smem + kc * 8192 + (i_local >> 3) * 1024 + (i_local & 7) * 128;
       const uint32_t sw = i_local & 7;
       const uint32_t sempty_leader = ptx::mapa(bar(B_SEMPTY), 0);
-      const uint32_t gfull_leader0 = ptx::mapa(bar(B_GFULL + kc), 0);
+      const uint32_t gfull_leader = ptx::mapa(bar(B_GFULL + kc), 0);
       const uint32_t accempty_leader = ptx::mapa(bar(B_ACCEMPTY), 0);
       uint32_t gs = 0;
 
@@ -491,10 +482,8 @@ bwd2_kernel(const __grid_constant__ CUtensorMap tmap_x,    // X  box {64, 64 row
               pk[16 * c + 2 * x4 + 1] = *reinterpret_cast<const uint32_t*>(&p1);
             }
           }
-          const uint32_t gb = g_buf(gs);
-          const uint32_t g_row = g_row0 + gb * G_BYTES;
-          ptx::mbar_wait(bar(B_GEMPTY + 4 * gb + kc), g_par(gs) ^ 1u);    // the gradient MMAs that last read this box are done
-          ptx::mbar_wait(bar(B_GSTORED + 4 * gb + kc), g_par(gs) ^ 1u);   // ... and so is its ring store
+          ptx::mbar_wait(bar(B_GEMPTY + kc), (gs & 1u) ^ 1u);    // the gradient MMAs that last read this box are done
+          ptx::mbar_wait(bar(B_GSTORED + kc), (gs & 1u) ^ 1u);   // ... and so is its ring store
 #pragma unroll
           for (int ch = 0; ch < 8; ++ch)
             pair::st_shared_v4(g_row + ((static_cast<uint32_t>(ch) ^ sw) << 4), pk[4 * ch], pk[4 * ch + 1], pk[4 * ch + 2],
@@ -502,8 +491,8 @@ bwd2_kernel(const __grid_constant__ CUtensorMap tmap_x,    // X  box {64, 64 row
           ptx::fence_proxy_async_smem();
           __syncwarp();
           if (lane == 0) {
-            ptx::mbar_arrive_cluster(gfull_leader0 + 32u * gb);
-            ptx::mbar_arrive(bar(B_GSFULL + 4 * gb + kc));
+            ptx::mbar_arrive_cluster(gfull_leader);
+            ptx::mbar_arrive(bar(B_GSFULL + kc));
           }
         }
 
@@ -572,12 +561,8 @@ bwd2_kernel(const __grid_constant__ CUtensorMap tmap_x,    // X  box {64, 64 row
                     const uint32_t st = ring_c + stage * C_STAGE;
                     const int grow = (slot * p.P + pp) * 128 + 64 * kb;
                     const int xrow = (sub.rb_lo + pp - sub.p_lo) * 128 + 64 * kb;
-                    for (int gi = 0; gi < 2; ++gi) {
-                      if (p.l2_hints)
-                        ptx::tma_load_2d_pair_hint(st + gi * 8192, &tmap_g, bar(B_FULL_A + stage), 128 * (int)rank + 64 * gi, grow, keep);
-                      else
-                        ptx::tma_load_2d_pair(st + gi * 8192, &tmap_g, bar(B_FULL_A + stage), 128 * (int)rank + 64 * gi, grow);
-                    }
+                    for (int gi = 0; gi < 2; ++gi)
+                      ptx::tma_load_2d_pair_hint(st + gi * 8192, &tmap_g, bar(B_FULL_A + stage), 128 * (int)rank + 64 * gi, grow, keep);
                     for (int gi = 0; gi < ngr; ++gi)
                       ptx::tma_load_2d_pair(st + 16384 + gi * 8192, &tmap_x, bar(B_FULL_A + stage),
                                             256 * hh + (wq >> 1) * (int)rank + 64 * gi, xrow);

@@ -18,8 +18,8 @@
 // In MODE 1 the gradient tile is rounded to bf16, written to shared memory as the K-major B operand
 // of a second MMA and contracted against the TRANSPOSED streamed operand:
 //       dXhat^T[d (128 lanes, nq chunks), i (BLOCK_I columns)] += Y^T[d, j] . G^T[j, i]  (UMMA 128 x BLOCK_I x 16)
-// The accumulators (nq * BLOCK_I TMEM columns) stay resident for the whole sweep; the S buffer(s) use
-// the remaining columns: BLOCK_I = 96 with one S buffer when d <= 512, else 64 with two.  Every MMA
+// The accumulators (nq * BLOCK_I TMEM columns) stay resident for the whole sweep; two S buffers use
+// the remaining columns: BLOCK_I = 64 (6 x 64 + 2 x 64 = 512 columns at d = 768).  Every MMA
 // operand is the same canonical layout: K-major, 128-byte rows, SWIZZLE_128B (what a TMA box
 // {64 elems, R rows} writes), so one descriptor builder serves all of them.
 //
@@ -55,7 +55,6 @@ constexpr float LOG2E = 1.4426950408889634f;
 constexpr float LN2 = 0.6931471805599453f;
 __host__ __device__ constexpr int small_bytes(int mode) { return mode == 1 ? 1536 : 3584; }  // barriers, tmem ptr, u/rinv, scratch
 __host__ __device__ constexpr int g_bytes(int block_i) { return block_i * BLOCK_J * 2; }     // bf16 gradient tile [i][128 j]
-__host__ __device__ constexpr int num_s_buffers(int mode, int block_i) { return (mode == 1 && block_i > 64) ? 1 : 2; }
 
 struct Params {
   int n_rows, n_cols, d;
@@ -143,12 +142,11 @@ template <int MODE, int BLOCK_I>
 __global__ void __launch_bounds__(num_threads(MODE, BLOCK_I), 1)
 clip_tc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__ CUtensorMap tmap_y,
                const __grid_constant__ CUtensorMap tmap_yt, const Params p) {
-  static_assert(BLOCK_I == 64 || BLOCK_I == 96 || BLOCK_I == 128, "BLOCK_I");
-  static_assert(MODE == 1 || BLOCK_I != 96, "forward uses 64 or 128 rows per CTA");
-  static_assert(MODE == 0 || BLOCK_I != 128, "backward: accumulators + logits must fit 512 TMEM columns");
+  static_assert(BLOCK_I == 64 || BLOCK_I == 128, "BLOCK_I");
+  static_assert(MODE == 0 || BLOCK_I == 64, "backward: accumulators + logits must fit 512 TMEM columns");
   constexpr int X_CHUNK = BLOCK_I * 128;        // bytes of one [BLOCK_I rows x 64 k] chunk of the resident panel
   constexpr int HALF = BLOCK_I / 2;             // TMEM columns per epilogue warp
-  constexpr int NSBUF = num_s_buffers(MODE, BLOCK_I);
+  constexpr int NSBUF = 2;
   constexpr int S_COL0 = (MODE == 0) ? 0 : TMEM_COLS - NSBUF * BLOCK_I;
   constexpr int G_BYTES = g_bytes(BLOCK_I);
   constexpr int NUM_EPI_WARPS = num_epi_warps(MODE, BLOCK_I);

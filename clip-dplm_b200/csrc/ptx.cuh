@@ -69,37 +69,16 @@ __device__ __forceinline__ void tma_load_2d(uint32_t dst_smem, const CUtensorMap
       : "memory");
 }
 
-// Same, multicast to every CTA of the cluster whose bit is set in `mask`: the box lands at the same
-// CTA-relative offset in each destination and signals the mbarrier at the same offset there.
-__device__ __forceinline__ void tma_load_2d_mc(uint32_t dst_smem, const CUtensorMap* m, uint32_t bar, int c0, int c1,
-                                               uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(dst_smem), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
-
-// 2-D tiled store shared -> global (bulk async-group completion).  The box is read from shared memory through the async
-// proxy: generic-proxy writes to it need fence.proxy.async first; the source may be reused after wait_group.read.
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* m, uint32_t src_smem, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
-               ::"l"(reinterpret_cast<uint64_t>(m)), "r"(src_smem), "r"(c0), "r"(c1)
-               : "memory");
-}
-// L2 eviction-priority policies for TMA traffic (createpolicy): evict_last keeps a producer/consumer ring resident until its
-// slots are overwritten (dirty lines that are evicted early cost a DRAM write-back each), evict_first marks streams that
-// are dead after use.
+// L2 eviction-priority policy for TMA traffic (createpolicy): evict_last keeps a producer/consumer ring resident until its
+// slots are overwritten (dirty lines that are evicted early cost a DRAM write-back each).
 __device__ __forceinline__ uint64_t l2_policy_evict_last() {
   uint64_t pol;
   asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
   return pol;
 }
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
+// 2-D tiled store shared -> global (bulk async-group completion) with an L2 cache policy.  The box is read from shared
+// memory through the async proxy: generic-proxy writes to it need fence.proxy.async first; the source may be reused after
+// wait_group.read.
 __device__ __forceinline__ void tma_store_2d_hint(const CUtensorMap* m, uint32_t src_smem, int c0, int c1, uint64_t policy) {
   asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group.L2::cache_hint [%0, {%2, %3}], [%1], %4;"
                ::"l"(reinterpret_cast<uint64_t>(m)), "r"(src_smem), "r"(c0), "r"(c1), "l"(policy)
@@ -183,12 +162,6 @@ __device__ __forceinline__ void mma_f16(uint32_t d_tmem, uint64_t a_desc, uint64
 // Implies tcgen05.fence::before_thread_sync.
 __device__ __forceinline__ void mma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-
-// Same, arriving on the barrier at this offset in every CTA of the cluster selected by `mask`.
-__device__ __forceinline__ void mma_commit_mc(uint32_t bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(bar), "h"(mask) : "memory");
 }
 
 // Software-pipelined issue blocks.  An mbarrier.try_wait costs ~170 clk even when the phase has already
@@ -288,24 +261,6 @@ __device__ __forceinline__ uint32_t mapa(uint32_t addr, uint32_t rank) {
 __device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
   asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
 }
-__device__ __forceinline__ bool mbar_try_wait_cluster(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred P;\n\t"
-      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 P, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, P;\n\t}"
-      : "=r"(ok)
-      : "r"(bar), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-// wait on a LOCAL barrier whose arrivals may come from the peer CTA (acquire at cluster scope)
-__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {
-  uint32_t spins = 0;
-  while (!mbar_try_wait_cluster(bar, parity)) {
-    if (++spins > (1u << 26)) __trap();
-  }
-}
 __device__ __forceinline__ void tmem_alloc_pair(uint32_t dst_smem, uint32_t ncols) {   // same warp id in both CTAs
   asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem), "r"(ncols) : "memory");
   asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
@@ -328,21 +283,6 @@ __device__ __forceinline__ void tma_load_2d_pair_hint(uint32_t dst_smem, const C
       " [%0], [%1, {%3, %4}], [%2], %5;"
       ::"r"(dst_smem), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar & 0xFEFFFFFFu), "r"(c0), "r"(c1), "l"(policy)
       : "memory");
-}
-// The same box multicast into every CTA of the cluster whose bit is set in `mask` (same CTA-relative offset); each
-// destination counts the bytes on ITS pair leader's mbarrier (peer bit cleared, as in tma_load_2d_pair).
-__device__ __forceinline__ void tma_load_2d_pair_mc(uint32_t dst_smem, const CUtensorMap* m, uint32_t bar, int c0, int c1,
-                                                    uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(dst_smem), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar & 0xFEFFFFFFu), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
-// commit arriving on the barrier at this offset in the CTAs of `mask`
-__device__ __forceinline__ void mma_commit_pair_mask(uint32_t bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(bar), "h"(mask) : "memory");
 }
 // arrive on the barrier at this offset in BOTH CTAs once every tcgen05.mma issued so far by this thread has completed
 __device__ __forceinline__ void mma_commit_pair(uint32_t bar) {

@@ -397,11 +397,11 @@ class CudaEngine:
         _lib.check(self.lib.clipnce_link_barrier(peers, world, rank, phase, _stream()), "link_barrier")
 
     @_guard
-    def link_push_rows(self, x, c_dtype, peers, world, rank, rows_off, rinv_off, row0, max_blocks=0):
+    def link_push_rows(self, x, c_dtype, peers, world, rank, rows_off, rinv_off, row0):
         self._chk(x, (torch.bfloat16, torch.float32), "embedding")
         n, d = x.shape
         _lib.check(self.lib.clipnce_link_push_rows(_p(x), _DT[x.dtype], n, d, _DT[c_dtype], peers, world, rank, rows_off,
-                                                   rinv_off, row0, max_blocks, _stream()), "link_push_rows")
+                                                   rinv_off, row0, _stream()), "link_push_rows")
 
     @_guard
     def link_copy(self, src, peers, world, rank, dst_off):

@@ -28,18 +28,11 @@ import torch.distributed as dist
 
 PHASE_COLS, PHASE_STATS, PHASE_LOSS, PHASE_CLOSE, PHASE_GRADS, PHASE_BLOCKS = 0, 1, 2, 3, 4, 5
 # The B rows travel BESIDE the forward sweep (copy engines + per-block flags, PeerExchange.gather_cols_beside) where the
-# forward kernel can wait block by block; CLIPNCE_GATHER_BESIDE=0 keeps the push kernel + barrier in front of the sweep.
-GATHER_BESIDE = os.environ.get("CLIPNCE_GATHER_BESIDE", "1") not in ("", "0")
-# ... and where the sweep is long enough to hide the delivery chain (world - 1 blocks, each two copy-engine transfers and a
-# flag kernel, ~25 us per block): measured on 8 GPUs, 8192 local rows x 65536 columns x 512 gain 4.4 % of the step, 4096
-# local rows x 32768 x 768 (a 190 us sweep) lose 8 %
+# forward kernel can wait block by block and the sweep is long enough to hide the delivery chain (world - 1 blocks, each
+# two copy-engine transfers and a flag kernel, ~25 us per block): measured on 8 GPUs, 8192 local rows x 65536 columns x 512
+# gain 4.4 % of the step, 4096 local rows x 32768 x 768 (a 190 us sweep) lose 8 %.  Below this the push kernel + barrier
+# run in front of the sweep.  CLIPNCE_GATHER_BESIDE_MIN_ROWS: test hook.
 GATHER_BESIDE_MIN_ROWS = int(os.environ.get("CLIPNCE_GATHER_BESIDE_MIN_ROWS", "8192"))
-# The A rows travel beside the forward sweep.  Every SM a push kernel takes costs the sweep a CTA-pair slot and -- its grid
-# being sized in whole waves of slots -- part of an extra wave (a full-grid push: 365 -> 435 us on 8 GPUs; 8 fat blocks:
-# +20 us on 8 GPUs, +80 us on 2 and 4), so by default the copy engines move them (CLIPNCE_LINK_BG=kernel for the push kernel
-# with BACKGROUND_BLOCKS blocks of 1024 threads).
-BACKGROUND_COPY_ENGINE = os.environ.get("CLIPNCE_LINK_BG", "copy").lower() != "kernel"
-BACKGROUND_BLOCKS = int(os.environ.get("CLIPNCE_LINK_BG_BLOCKS", "8"))
 
 
 def _all_gather(x, group):
@@ -209,16 +202,14 @@ class PeerExchange:
         cur = torch.cuda.current_stream()
         self.side.wait_stream(cur)          # behind barrier 0: the columns have the links to themselves
         lo = self.rank * self.n
+        # the rows already exist in the compute type (a_c) and their norms too: nothing to compute, so the copy engines
+        # move them and the forward sweep keeps every SM (a push kernel beside the sweep takes CTA-pair slots from it and
+        # part of an extra wave: a full-grid push 365 -> 435 us on 8 GPUs, 8 blocks of 1024 threads +20 us on 8, +80 us on
+        # 2 and 4 GPUs)
+        esz = a_c.element_size()
         with torch.cuda.stream(self.side):
-            if BACKGROUND_COPY_ENGINE:
-                # the rows already exist in the compute type (a_c) and their norms too: nothing to compute, so the
-                # copy engines move them and the forward sweep keeps every SM
-                esz = a_c.element_size()
-                self.engine.link_copy(a_c, self.peers, self.world, self.rank, self.o_xa + lo * self.d * esz)
-                self.engine.link_copy(rinv_a, self.peers, self.world, self.rank, self.o_rinv_xa + lo * 4)
-            else:
-                self.engine.link_push_rows(a, compute_dtype, self.peers, self.world, self.rank, self.o_xa, self.o_rinv_xa,
-                                           lo, max_blocks=BACKGROUND_BLOCKS)
+            self.engine.link_copy(a_c, self.peers, self.world, self.rank, self.o_xa + lo * self.d * esz)
+            self.engine.link_copy(rinv_a, self.peers, self.world, self.rank, self.o_rinv_xa + lo * 4)
         self._side_busy = True
 
     def gather_rows_end(self):

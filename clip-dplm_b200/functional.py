@@ -243,7 +243,7 @@ def fused_clip_loss(a, b, logit_scale, *, symmetric: bool = True, scale_is_log: 
 # ------------------------------------------------------------------------------------------------------------------------
 def _no_group():
     import os
-    return os.environ.get("CLIPNCE_NO_GROUP", "0") not in ("", "0")     # A/B and test hook: pair steps only
+    return os.environ.get("CLIPNCE_NO_GROUP", "0") not in ("", "0")     # test hook: pair steps only
 
 
 GROUP_MAX_ROWS = 8192     # measured (tools/bench_trimodal.py): 3.4x at N = 1024, 1.43x at 4096, 0.92x at 8192 against three pair steps

@@ -96,7 +96,7 @@ def contrastive_forward(engine, a, b, scale, *, symmetric=True, extra=None, grou
             scale = scale()
         # the gather runs BESIDE the forward sweep where the sweep can wait block by block (include/clipnce.h,
         # clipnce_forward_gathered): every rank decides from the same shapes, types and scale hint
-        beside = bool(_exchange.GATHER_BESIDE and getattr(xchg, "kind", "") == "nvlink-peer" and extra is None
+        beside = bool(getattr(xchg, "kind", "") == "nvlink-peer" and extra is None
                       and b.dtype == compute_dtype == torch.bfloat16 and n_local % 256 == 0
                       and n_local >= _exchange.GATHER_BESIDE_MIN_ROWS and n_global <= (1 << 22)
                       and hasattr(engine, "forward_gathered") and engine.forward_gathered_ok(compute_dtype, d, scale, flags))

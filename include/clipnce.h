@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define CLIPNCE_VERSION 108
+#define CLIPNCE_VERSION 109
 
 /* element types */
 #define CLIPNCE_BF16 0
@@ -352,12 +352,10 @@ int clipnce_link_barrier(void* const* peer_base, int world, int rank, int phase,
 /* Fused F.normalize row norms + all-gather: x [n,d] (in_dtype) -> rinv_i = 1 / max(|x_i|, 1e-12) and the rows,
  * converted to c_dtype, are stored into EVERY rank's buffer: rows at rows_offset + (row0 + i) * d * sizeof(c_dtype),
  * rinv at rinv_offset + (row0 + i) * 4.  row0 = rank * n.  Publish with clipnce_link_barrier.
- * max_blocks = 0: the whole GPU pushes (nothing else is running: the columns, before the forward sweep);
- * max_blocks > 0: at most that many thread blocks -- the background variant for rows that travel beside a contraction
- * kernel (the A rows, needed by the backward only), which then loses that many SMs at most. */
+ * The push takes the whole GPU: issue it where nothing else runs (the columns, before the forward sweep); rows that
+ * travel beside a contraction kernel go by clipnce_link_copy. */
 int clipnce_link_push_rows(const void* x, int in_dtype, int64_t n, int64_t d, int c_dtype, void* const* peer_base,
-                           int world, int rank, int64_t rows_offset, int64_t rinv_offset, int64_t row0, int max_blocks,
-                           void* stream);
+                           int world, int rank, int64_t rows_offset, int64_t rinv_offset, int64_t row0, void* stream);
 
 /* Copy `bytes` from src to byte offset dst_offset of every rank's buffer with the COPY ENGINES (cudaMemcpyAsync per
  * peer, no SM involved): the background gather of rows that travel beside a contraction kernel -- the A rows, read by

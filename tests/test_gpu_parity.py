@@ -565,3 +565,22 @@ def test_speculative_large_scale_forward_and_its_exact_fallback(monkeypatch, n, 
     assert abs(dt - float(ref["d_logit_scale"])) <= GRAD_RTOL_BF16 * abs(float(ref["d_logit_scale"])) + 1e-7
     if flip != "none":    # the flipped entries decide the loss: it is ~ 2 s cos / n per entry, far from the unflipped value
         assert float(ref["loss"]) > 0.05
+
+
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two CUDA devices")
+def test_second_device_in_one_process():
+    """The kernels' shared-memory limit is raised per device: one process that runs the loss on cuda:0 and then on cuda:1
+    (16384 x 512: the pair forward and the two-sided backward) gets the same loss and gradients, bit for bit, on both."""
+    from clip_dplm_b200 import fused_clip_loss
+    a, b = O.make_inputs(16384, 512, seed=41)
+    outs = []
+    for dev in ("cuda:0", "cuda:1"):
+        ac = a.to(dev).bfloat16().requires_grad_(True)
+        bc = b.to(dev).bfloat16().requires_grad_(True)
+        t = torch.tensor(O.LOGIT_SCALE_INIT, device=dev, requires_grad=True)
+        loss = fused_clip_loss(ac, bc, t)
+        loss.backward()
+        torch.cuda.synchronize(dev)
+        outs.append([x.detach().cpu() for x in (loss, ac.grad, bc.grad, t.grad)])
+    for x0, x1 in zip(*outs):
+        assert torch.equal(x0, x1)

@@ -38,7 +38,6 @@ one(512, 256, 1 / 0.07, "two-sweep, split sweep", CLIPNCE_NO_BWD2="1", CLIPNCE_S
 one(512, 256, 100.0, "family 2, speculative forward")
 one(512, 256, 100.0, "family 2, exact online sweeps", CLIPNCE_NO_SPECULATE="1")
 one(1024, 256, 100.0, "family 2, two-sided backward", CLIPNCE_BWD2_P="5")
-one(1024, 512, 1 / 0.07, "two-sweep, 4-CTA multicast", CLIPNCE_NO_BWD2="1", CLIPNCE_BWD_MC="1")
 one(300, 192, 10.0, "single-CTA tcgen05 kernels")
 one(200, 100, 10.0, "exact CUDA-core kernels")
 # grouped launch: three pairs over three embeddings (tri-modal model), ragged rows

@@ -48,14 +48,11 @@ def main():
             n, d = (int(v) for v in shape.lower().split("x"))
             comm, scale, parity = "auto", 1 / 0.07, False
             os.environ.pop("CLIPNCE_E2E_SPLIT", None)
-            exchange.GATHER_BESIDE = True
             for o in opts:
                 if o in ("auto", "link", "nccl"):
                     comm = o
                 elif o == "parity":
                     parity = True
-                elif o in ("beside", "nobeside"):   # gather of the columns beside the forward sweep, or push + barrier before it
-                    exchange.GATHER_BESIDE = o == "beside"
                 elif o in ("split", "nosplit"):     # host-fed (e2e) step as forward graph + backward graph, or as one graph
                     os.environ["CLIPNCE_E2E_SPLIT"] = "1" if o == "split" else "0"
                 elif o.startswith("s"):
