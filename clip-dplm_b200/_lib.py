@@ -42,10 +42,9 @@ SIGNATURES = {
                             _int, _int, _vp, _int, _vp, _vp, _int, _vp, _vp, _sz, _vp],
     "clipnce_backward_both_workspace_bytes": [_i64, _i64, _i64, _int, _f32, _int, _int, ctypes.POINTER(_sz)],
     "clipnce_backward_both_sharded": [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _f32, _vp, _vp, _vp, _vp, _vp, _f32, _int, _int,
-                                      _vp, _int, _vp, _vp, _int, _vp, ctypes.POINTER(_vp), _int, _int, _i64, _vp, _sz, _vp],
+                                      ctypes.POINTER(_vp), _int, _int, _i64, _vp, _sz, _vp],
     "clipnce_finish_sharded": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _int, _f32, _int, _int, _int, _int,
-                               _vp, _vp, _vp, _sz, _vp],
-    "clipnce_finish_slots": [_vp, _int, _vp, _int, _vp, _int, _vp, _vp, _i64, _i64, _vp, _int, _vp],
+                               _int, _int, _vp, _vp, _vp, _sz, _vp],
     "clipnce_backward_both_dx": [_vp, _vp, _vp, _vp, _i64, _i64, _f32, _vp, _vp, _vp, _vp, _vp, _f32, _int, _int, _vp, _vp,
                                  _int, _vp, _vp, _vp, _int, _vp, _vp, _sz, _vp],
     "clipnce_group_workspace_bytes": [_int, _int, _i64, _i64, _int, _f32, _int, ctypes.POINTER(_sz)],
@@ -130,7 +129,7 @@ def load():
             fn = getattr(lib, name)          # AttributeError here == header/library mismatch
             fn.argtypes = argtypes
             fn.restype = _RESTYPES.get(name, ctypes.c_int)
-        if lib.clipnce_version() != 109:
+        if lib.clipnce_version() != 110:
             raise RuntimeError("clip_dplm_b200: libclipnce.so version mismatch; rebuild")
         _lib = lib
         return lib

@@ -588,6 +588,45 @@ struct Deferred {
   bool ds_pending = false;
 };
 
+// A side of the finishing pass with one contribution of n_split slabs of [n, d].
+aux::FinishSide finish_side(const float* parts, int n_split, int64_t n, int64_t d, const void* xc, const void* xo,
+                            const float* rinv, void* dx, float* ds_part) {
+  aux::FinishSide s;
+  memset(&s, 0, sizeof s);
+  s.parts[0] = parts; s.n_contrib = 1; s.n_split = n_split; s.slab = n * d; s.n = n;
+  s.xc = xc; s.xo = xo; s.rinv = rinv; s.dx = dx; s.ds_part = ds_part;
+  return s;
+}
+
+template <typename TC, typename TI, typename TO>
+void finish_kernel(const aux::FinishSides& fs, dim3 grid, size_t smem, bool v4, const float* grad_scale, int d, cudaStream_t st) {
+  if (v4) aux::finish_rows<TC, TI, TO, 4><<<grid, 256, smem, st>>>(fs, grad_scale, d);
+  else aux::finish_rows<TC, TI, TO, 1><<<grid, 256, smem, st>>>(fs, grad_scale, d);
+}
+
+// ONE launch of the finishing pass over sides[0, n_sides), each of at most n rows, all of the same types: the compute
+// type `dtype` (xc), the caller's rows `in_dtype` (xo), the gradient `out_dtype` (dx).  v4: 16-byte accesses (d % 4 == 0,
+// every row base 4-element aligned).  8 d floats of shared memory per block: d <= 1536.
+int launch_finish(const aux::FinishSide* sides, int n_sides, int64_t n, int64_t d, int dtype, int in_dtype, int out_dtype,
+                  const float* grad_scale, bool v4, cudaStream_t st) {
+  aux::FinishSides fs;
+  memset(&fs, 0, sizeof fs);
+  for (int i = 0; i < n_sides; ++i) fs.s[i] = sides[i];
+  const dim3 grid((unsigned)ceil_div(n, 8), (unsigned)n_sides);
+  const size_t smem = sizeof(float) * 8 * (size_t)d;
+  const int di = (int)d;
+  using bf = __nv_bfloat16;
+  const bool ib = in_dtype == CLIPNCE_BF16, ob = out_dtype == CLIPNCE_BF16;
+  if (dtype == CLIPNCE_BF16 && ib && ob) finish_kernel<bf, bf, bf>(fs, grid, smem, v4, grad_scale, di, st);
+  else if (dtype == CLIPNCE_BF16 && ib) finish_kernel<bf, bf, float>(fs, grid, smem, v4, grad_scale, di, st);
+  else if (dtype == CLIPNCE_BF16 && ob) finish_kernel<bf, float, bf>(fs, grid, smem, v4, grad_scale, di, st);
+  else if (dtype == CLIPNCE_BF16) finish_kernel<bf, float, float>(fs, grid, smem, v4, grad_scale, di, st);
+  else if (ob) finish_kernel<float, float, bf>(fs, grid, smem, v4, grad_scale, di, st);
+  else finish_kernel<float, float, float>(fs, grid, smem, v4, grad_scale, di, st);
+  CUDA_TRY(cudaGetLastError());
+  return 0;
+}
+
 int backward_impl(const void* x, const void* y, const void* y_t, int64_t ld_t, const float* rinv_x,
                   const float* rinv_y, int64_t n_rows, int64_t n_cols, int64_t d, int64_t diag_offset, float scale,
                   const float* scale_dev, const float* row_m, const float* row_w, const float* col_m, const float* col_w, float diag_w,
@@ -755,30 +794,11 @@ int clipnce_backward_dx(const void* x, const void* y, const void* y_t, int64_t l
     return clipnce_normalize_backward(x_orig, in_dtype, rinv_x, dx_hat, grad_scale, n_rows, d, dx, out_dtype, stream);
   }
   float* ds_part = df.ds_pending ? reinterpret_cast<float*>(workspace) : nullptr;   // [n_blk] at the workspace start
-  const int64_t slab_elems = n_rows * d;
-  const unsigned grid = (unsigned)n_blk;
   // 16-byte accesses when every row base is 4-element aligned (always so for the tensor-core path: d % 8 == 0)
   const bool v4 = d % 4 == 0 && (reinterpret_cast<uintptr_t>(x) & 15u) == 0 && (reinterpret_cast<uintptr_t>(x_orig) & 15u) == 0 &&
                   (reinterpret_cast<uintptr_t>(dx) & 15u) == 0 && (reinterpret_cast<uintptr_t>(df.parts) & 15u) == 0;
-#define FINISH(TC, TI, TO)                                                                                                 \
-  do {                                                                                                                     \
-    if (v4)                                                                                                                \
-      aux::finish_rows_v4<TC, TI, TO><<<grid, 256, smem, st>>>(df.parts, df.n_split, slab_elems, (const TC*)x,             \
-                                                               (const TI*)x_orig, rinv_x, grad_scale, n_rows, di, (TO*)dx, \
-                                                               ds_part);                                                   \
-    else                                                                                                                   \
-      aux::finish_rows<TC, TI, TO><<<grid, 256, smem, st>>>(df.parts, df.n_split, slab_elems, (const TC*)x,                \
-                                                            (const TI*)x_orig, rinv_x, grad_scale, n_rows, di, (TO*)dx,    \
-                                                            ds_part);                                                      \
-  } while (0)
-  if (dtype == CLIPNCE_BF16 && in_dtype == CLIPNCE_BF16 && out_dtype == CLIPNCE_BF16) FINISH(__nv_bfloat16, __nv_bfloat16, __nv_bfloat16);
-  else if (dtype == CLIPNCE_BF16 && in_dtype == CLIPNCE_BF16) FINISH(__nv_bfloat16, __nv_bfloat16, float);
-  else if (dtype == CLIPNCE_BF16 && out_dtype == CLIPNCE_BF16) FINISH(__nv_bfloat16, float, __nv_bfloat16);
-  else if (dtype == CLIPNCE_BF16) FINISH(__nv_bfloat16, float, float);
-  else if (out_dtype == CLIPNCE_BF16) FINISH(float, float, __nv_bfloat16);
-  else FINISH(float, float, float);
-#undef FINISH
-  CUDA_TRY(cudaGetLastError());
+  const aux::FinishSide side = finish_side(df.parts, df.n_split, n_rows, d, x, x_orig, rinv_x, dx, ds_part);
+  if ((rc = launch_finish(&side, 1, n_rows, d, dtype, in_dtype, out_dtype, grad_scale, v4, st))) return rc;
   if (df.ds_pending) {
     aux::reduce_scalar_partials_par<<<1, 256, 0, st>>>(ds_part, (int)n_blk, 1.f, d_scale_sum);
     CUDA_TRY(cudaGetLastError());
@@ -803,8 +823,8 @@ struct GroupPlan {
 
 int group_plan(int n_members, int n_prob, int64_t n, int64_t d, int dtype, float scale, int flags, GroupPlan* pl) {
   memset(pl, 0, sizeof *pl);
-  if (n_members < 1 || n_members > aux::FG_MEMBERS || n_prob < 1 || 2 * n_prob > pair::MAX_GROUP || n < 1 || d < 1)
-    return fail(CLIPNCE_EINVAL, "group: 1..%d members, 1..%d problems", aux::FG_MEMBERS, pair::MAX_GROUP / 2);
+  if (n_members < 1 || n_members > aux::FINISH_SIDES || n_prob < 1 || 2 * n_prob > pair::MAX_GROUP || n < 1 || d < 1)
+    return fail(CLIPNCE_EINVAL, "group: 1..%d members, 1..%d problems", aux::FINISH_SIDES, pair::MAX_GROUP / 2);
   pl->fam = tc_family(dtype, d, scale, flags);
   if (!((pl->fam == 1 && pair_eligible(d)) || pl->fam == 2) || (flags & CLIPNCE_FLAG_UNBOUNDED)) { pl->fam = 0; return 0; }
   pl->rows = d <= 512 ? 128 : 64;
@@ -1005,34 +1025,30 @@ int clipnce_group_backward(const void* stack, const float* rinv, int n_members, 
   p.grp.n_prob = 2 * n_prob; p.grp.pairs_per_prob = pl.bwd_pairs; p.grp.steps_per_prob = pl.steps; p.grp.n_valid = (int)n;
   p.grp.stack_rows = (int)(n_members * pl.n_pad);
   p.grp.gscale = grad_scale; p.grp.gmod = n_prob;
-  aux::FinishGroup fg;
-  memset(&fg, 0, sizeof fg);
-  fg.n_pad = pl.n_pad; fg.n_valid = n;
+  // the finishing pass, one side per member: the gradient of member m's normalised rows is the sum of the slabs of every
+  // virtual problem in which m was the resident operand (its X sides and its Y sides).  Every pair's sum G.S appears once
+  // per side in the row dots: reduce_group_scalars halves it.
+  aux::FinishSide sides[aux::FINISH_SIDES];
+  memset(sides, 0, sizeof sides);
+  for (int m = 0; m < n_members; ++m) {
+    aux::FinishSide& s = sides[m];
+    s.n_split = pl.bwd_n_split; s.slab = 2 * V * d; s.row0 = m * pl.n_pad; s.n = n;
+    s.xc = stack; s.xo = stack_orig; s.rinv = rinv; s.dx = d_stack;
+    s.ds_part = ds_part + (size_t)m * pl.n_blk; s.sq_part = sq_part + (size_t)m * pl.n_blk;
+  }
   for (int k = 0; k < 2 * n_prob; ++k) {
     const int q = k % n_prob;
     const int res = k < n_prob ? x_member[q] : y_member[q], str = k < n_prob ? y_member[q] : x_member[q];
     p.grp.xshift[k] = (int)((res - k) * pl.n_pad);
     p.grp.yshift[k] = (int)((str - k) * pl.n_pad);
     p.grp.cshift[k] = (int)(k < n_prob ? V : -V);
-    if (fg.n_contrib[res] >= aux::FG_CONTRIB) return fail(CLIPNCE_EINVAL, "group_backward: too many problems share member %d", res);
-    fg.vprob[res][fg.n_contrib[res]++] = k;
+    aux::FinishSide& s = sides[res];
+    if (s.n_contrib >= aux::FINISH_CONTRIB) return fail(CLIPNCE_EINVAL, "group_backward: too many problems share member %d", res);
+    s.parts[s.n_contrib++] = slabs + (size_t)k * pl.n_pad * d;
   }
   if ((rc = pl.fam == 2 ? launch_pair_bwd<true>(stack, stack, p, st) : launch_pair_bwd<false>(stack, stack, p, st))) return rc;
 
-  const int di = (int)d;
-  const size_t smem = sizeof(float) * 8 * (size_t)d;
-  const dim3 grid((unsigned)pl.n_blk, (unsigned)n_members);
-  const int64_t slab_elems = 2 * V * d;
-#define FINISH_G(TI, TO)                                                                                                  \
-  aux::finish_rows_group<__nv_bfloat16, TI, TO><<<grid, 256, smem, st>>>(slabs, pl.bwd_n_split, slab_elems, fg,          \
-                                                                        (const __nv_bfloat16*)stack, (const TI*)stack_orig, \
-                                                                        rinv, di, (TO*)d_stack, ds_part, sq_part)
-  if (in_dtype == CLIPNCE_BF16 && out_dtype == CLIPNCE_BF16) FINISH_G(__nv_bfloat16, __nv_bfloat16);
-  else if (in_dtype == CLIPNCE_BF16) FINISH_G(__nv_bfloat16, float);
-  else if (out_dtype == CLIPNCE_BF16) FINISH_G(float, __nv_bfloat16);
-  else FINISH_G(float, float);
-#undef FINISH_G
-  CUDA_TRY(cudaGetLastError());
+  if ((rc = launch_finish(sides, n_members, pl.n_pad, d, CLIPNCE_BF16, in_dtype, out_dtype, nullptr, true, st))) return rc;
   if (d_scale_sum || grad_sumsq) {
     aux::reduce_group_scalars<<<1 + n_members, 256, 0, st>>>(ds_part, sq_part, n_members, pl.n_blk, d_scale_sum, grad_sumsq);
     CUDA_TRY(cudaGetLastError());
@@ -1150,25 +1166,6 @@ bool bwd2_plan(int64_t n_rows, int64_t n_cols, int64_t d, int dtype, float scale
   return true;
 }
 
-// One pass over the fp32 gradient of normalised rows: sum of n_split slabs + row dots (sum G.S) + normalise backward.
-int launch_finish(const float* parts, int n_split, int64_t slab_elems, const void* xc, const void* xo, int in_dtype,
-                  const float* rinv, const float* grad_scale, int64_t n, int64_t d, void* dx, int out_dtype, float* ds_part,
-                  cudaStream_t st) {
-  const unsigned grid = (unsigned)ceil_div(n, 8);
-  const size_t smem = sizeof(float) * 8 * (size_t)d;
-  const int di = (int)d;
-#define FINISH3(TI, TO)                                                                                                \
-  aux::finish_rows_v4<__nv_bfloat16, TI, TO><<<grid, 256, smem, st>>>(parts, n_split, slab_elems, (const __nv_bfloat16*)xc, \
-                                                                      (const TI*)xo, rinv, grad_scale, n, di, (TO*)dx, ds_part)
-  if (in_dtype == CLIPNCE_BF16 && out_dtype == CLIPNCE_BF16) FINISH3(__nv_bfloat16, __nv_bfloat16);
-  else if (in_dtype == CLIPNCE_BF16) FINISH3(__nv_bfloat16, float);
-  else if (out_dtype == CLIPNCE_BF16) FINISH3(float, __nv_bfloat16);
-  else FINISH3(float, float);
-#undef FINISH3
-  CUDA_TRY(cudaGetLastError());
-  return 0;
-}
-
 int bwd2_launch(const Bwd2Plan& pl, const void* x, const void* y, const float* rinv_x, const float* rinv_y, int64_t n_rows,
                 int64_t n_cols, int64_t d, int64_t diag_offset, float scale, const float* scale_dev, const float* row_m,
                 const float* row_w, const float* col_m, const float* col_w, float diag_w, char* ws, float* const* dy_peer,
@@ -1242,12 +1239,11 @@ int clipnce_backward_both_dx(const void* x, const void* y, const float* rinv_x, 
     return rc;
   // tails: segment sum + row dots (sum G.S, side A only) + normalise backward, one pass per side
   float* ds_part = reinterpret_cast<float*>(ws + pl.off_part);
-  if ((rc = launch_finish(reinterpret_cast<float*>(ws + pl.off_dxh), pl.n_seg, n * d, x, x_orig, in_dtype, rinv_x, grad_scale, n, d,
-                          dx, out_dtype, d_scale_sum ? ds_part : nullptr, st)))
-    return rc;
-  if ((rc = launch_finish(reinterpret_cast<float*>(ws + pl.off_dyh), 1, n * d, y, y_orig, in_dtype, rinv_y, grad_scale, n, d, dy,
-                          out_dtype, nullptr, st)))
-    return rc;
+  const aux::FinishSide sx = finish_side(reinterpret_cast<float*>(ws + pl.off_dxh), pl.n_seg, n, d, x, x_orig, rinv_x, dx,
+                                         d_scale_sum ? ds_part : nullptr);
+  const aux::FinishSide sy = finish_side(reinterpret_cast<float*>(ws + pl.off_dyh), 1, n, d, y, y_orig, rinv_y, dy, nullptr);
+  if ((rc = launch_finish(&sx, 1, n, d, CLIPNCE_BF16, in_dtype, out_dtype, grad_scale, true, st))) return rc;
+  if ((rc = launch_finish(&sy, 1, n, d, CLIPNCE_BF16, in_dtype, out_dtype, grad_scale, true, st))) return rc;
   if (d_scale_sum) {
     aux::reduce_scalar_partials_par<<<1, 256, 0, st>>>(ds_part, (int)ceil_div(n, 8), 1.f, d_scale_sum);
     CUDA_TRY(cudaGetLastError());
@@ -1258,15 +1254,10 @@ int clipnce_backward_both_dx(const void* x, const void* y, const float* rinv_x, 
 int clipnce_backward_both_sharded(const void* x, const void* y, const float* rinv_x, const float* rinv_y, int64_t n_rows,
                                   int64_t n_cols, int64_t d, int64_t diag_offset, float scale, const float* scale_dev,
                                   const float* row_m, const float* row_w, const float* col_m, const float* col_w,
-                                  float diag_w, int dtype, int flags, const void* x_orig, int in_dtype,
-                                  const float* grad_scale, void* dx, int out_dtype, float* d_scale_sum,
-                                  void* const* peer_base, int world, int rank, int64_t slots_offset, void* workspace,
-                                  size_t workspace_bytes, void* stream) {
-  if (!x || !y || !rinv_x || !rinv_y || !row_m || !row_w || !col_m || !col_w || !x_orig || !workspace || !peer_base)
+                                  float diag_w, int dtype, int flags, void* const* peer_base, int world, int rank,
+                                  int64_t slots_offset, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!x || !y || !rinv_x || !rinv_y || !row_m || !row_w || !col_m || !col_w || !workspace || !peer_base)
     return fail(CLIPNCE_EINVAL, "backward_both_sharded: null pointer");
-  if ((in_dtype != CLIPNCE_BF16 && in_dtype != CLIPNCE_F32) || (out_dtype != CLIPNCE_BF16 && out_dtype != CLIPNCE_F32))
-    return fail(CLIPNCE_EINVAL, "backward_both_sharded: bad dtype");
-  if (in_dtype == dtype && x_orig != x) return fail(CLIPNCE_EINVAL, "backward_both_sharded: x_orig of the compute type must be x itself");
   if (!aligned16(x) || !aligned16(y) || !aligned16(workspace)) return fail(CLIPNCE_EINVAL, "backward_both_sharded: operands must be 16-byte aligned");
   if (world < 2 || world > pair2::MAX_WORLD || rank < 0 || rank >= world || slots_offset < 0 || slots_offset % 16 != 0)
     return fail(CLIPNCE_EINVAL, "backward_both_sharded: bad world / rank / slots_offset");
@@ -1277,37 +1268,27 @@ int clipnce_backward_both_sharded(const void* x, const void* y, const float* rin
   if (!bwd2_plan(n_rows, n_cols, d, dtype, scale, flags, world, &pl) || !bwd2_device_ok())
     return fail(CLIPNCE_EUNSUPPORTED, "backward_both_sharded: shape not served (see clipnce_backward_both_workspace_bytes)");
   if (workspace_bytes < pl.bytes) return fail(CLIPNCE_EWORKSPACE, "backward_both_sharded: workspace %zu < %zu", workspace_bytes, pl.bytes);
-  cudaStream_t st = as_stream(stream);
   char* ws = reinterpret_cast<char*>(workspace);
   float* dy_peer[pair2::MAX_WORLD];
   for (int s = 0; s < world; ++s) {   // this rank's slot in rank s's buffer: [n_rows, d] f32 (n_rows == columns per owner)
     if (!peer_base[s] || !aligned16(peer_base[s])) return fail(CLIPNCE_EINVAL, "backward_both_sharded: peer buffer %d is null or unaligned", s);
     dy_peer[s] = reinterpret_cast<float*>(reinterpret_cast<char*>(peer_base[s]) + slots_offset) + (size_t)rank * (size_t)n_rows * (size_t)d;
   }
-  if ((rc = bwd2_launch(pl, x, y, rinv_x, rinv_y, n_rows, n_cols, d, diag_offset, scale, scale_dev, row_m, row_w, col_m, col_w,
-                        diag_w, ws, dy_peer, world, st)))
-    return rc;
-  if (!dx) return 0;   // both tails are left to clipnce_finish_sharded (one launch for the two sides, behind the barrier)
-  float* ds_part = reinterpret_cast<float*>(ws + pl.off_part);
-  if ((rc = launch_finish(reinterpret_cast<float*>(ws + pl.off_dxh), pl.n_seg, n_rows * d, x, x_orig, in_dtype, rinv_x, grad_scale,
-                          n_rows, d, dx, out_dtype, d_scale_sum ? ds_part : nullptr, st)))
-    return rc;
-  if (d_scale_sum) {
-    aux::reduce_scalar_partials_par<<<1, 256, 0, st>>>(ds_part, (int)ceil_div(n_rows, 8), 1.f, d_scale_sum);
-    CUDA_TRY(cudaGetLastError());
-  }
-  return 0;
+  return bwd2_launch(pl, x, y, rinv_x, rinv_y, n_rows, n_cols, d, diag_offset, scale, scale_dev, row_m, row_w, col_m, col_w,
+                     diag_w, ws, dy_peer, world, as_stream(stream));
 }
 
 int clipnce_finish_sharded(const void* x, const void* x_orig, const float* rinv_x, void* dx, const void* y_local,
                            const void* y_orig, const float* rinv_y_local, void* dy, const float* slots, int64_t n_rows,
-                           int64_t n_cols, int64_t d, int dtype, float scale, int flags, int world, int in_dtype,
-                           int out_dtype, const float* grad_scale, float* d_scale_sum, void* workspace,
-                           size_t workspace_bytes, void* stream) {
+                           int64_t n_cols, int64_t d, int dtype, float scale, int flags, int world, int x_in_dtype,
+                           int x_out_dtype, int y_in_dtype, int y_out_dtype, const float* grad_scale, float* d_scale_sum,
+                           void* workspace, size_t workspace_bytes, void* stream) {
   if (!x || !x_orig || !rinv_x || !dx || !y_local || !y_orig || !rinv_y_local || !dy || !slots || !workspace)
     return fail(CLIPNCE_EINVAL, "finish_sharded: null pointer");
-  if ((in_dtype != CLIPNCE_BF16 && in_dtype != CLIPNCE_F32) || (out_dtype != CLIPNCE_BF16 && out_dtype != CLIPNCE_F32))
-    return fail(CLIPNCE_EINVAL, "finish_sharded: bad dtype");
+  for (int t : {x_in_dtype, x_out_dtype, y_in_dtype, y_out_dtype})
+    if (t != CLIPNCE_BF16 && t != CLIPNCE_F32) return fail(CLIPNCE_EINVAL, "finish_sharded: bad dtype");
+  if ((x_in_dtype == dtype && x_orig != x) || (y_in_dtype == dtype && y_orig != y_local))
+    return fail(CLIPNCE_EINVAL, "finish_sharded: x_orig / y_orig of the compute type must be x / y_local themselves");
   Bwd2Plan pl;
   if (!bwd2_plan(n_rows, n_cols, d, dtype, scale, flags, world, &pl))
     return fail(CLIPNCE_EUNSUPPORTED, "finish_sharded: shape not served by the two-sided backward");
@@ -1315,37 +1296,23 @@ int clipnce_finish_sharded(const void* x, const void* x_orig, const float* rinv_
   cudaStream_t st = as_stream(stream);
   char* ws = reinterpret_cast<char*>(workspace);
   float* ds_part = reinterpret_cast<float*>(ws + pl.off_part);
-  aux::FinishSide s0, s1;
-  s0.parts = reinterpret_cast<float*>(ws + pl.off_dxh); s0.n_split = pl.n_seg; s0.slab = n_rows * d; s0.xc = x; s0.xo = x_orig;
-  s0.rinv = rinv_x; s0.dx = dx; s0.ds_part = d_scale_sum ? ds_part : nullptr;
-  s1.parts = slots; s1.n_split = world; s1.slab = n_rows * d; s1.xc = y_local; s1.xo = y_orig; s1.rinv = rinv_y_local; s1.dx = dy;
-  s1.ds_part = nullptr;
-  const dim3 grid((unsigned)ceil_div(n_rows, 8), 2);
-  const size_t smem = sizeof(float) * 8 * (size_t)d;
-  const int di = (int)d;
-#define FINISHD(TI, TO) aux::finish_rows_v4_dual<__nv_bfloat16, TI, TO><<<grid, 256, smem, st>>>(s0, s1, grad_scale, n_rows, di)
-  if (in_dtype == CLIPNCE_BF16 && out_dtype == CLIPNCE_BF16) FINISHD(__nv_bfloat16, __nv_bfloat16);
-  else if (in_dtype == CLIPNCE_BF16) FINISHD(__nv_bfloat16, float);
-  else if (out_dtype == CLIPNCE_BF16) FINISHD(float, __nv_bfloat16);
-  else FINISHD(float, float);
-#undef FINISHD
-  CUDA_TRY(cudaGetLastError());
+  // side 0 sums the segment slabs of dA_hat, side 1 the ranks' slots of dB_hat; sides of the same types share ONE launch
+  // instead of queueing behind each other
+  const aux::FinishSide sides[2] = {
+      finish_side(reinterpret_cast<float*>(ws + pl.off_dxh), pl.n_seg, n_rows, d, x, x_orig, rinv_x, dx, d_scale_sum ? ds_part : nullptr),
+      finish_side(slots, world, n_rows, d, y_local, y_orig, rinv_y_local, dy, nullptr)};
+  int rc;
+  if (x_in_dtype == y_in_dtype && x_out_dtype == y_out_dtype) {
+    if ((rc = launch_finish(sides, 2, n_rows, d, CLIPNCE_BF16, x_in_dtype, x_out_dtype, grad_scale, true, st))) return rc;
+  } else {
+    if ((rc = launch_finish(&sides[0], 1, n_rows, d, CLIPNCE_BF16, x_in_dtype, x_out_dtype, grad_scale, true, st))) return rc;
+    if ((rc = launch_finish(&sides[1], 1, n_rows, d, CLIPNCE_BF16, y_in_dtype, y_out_dtype, grad_scale, true, st))) return rc;
+  }
   if (d_scale_sum) {
     aux::reduce_scalar_partials_par<<<1, 256, 0, st>>>(ds_part, (int)ceil_div(n_rows, 8), 1.f, d_scale_sum);
     CUDA_TRY(cudaGetLastError());
   }
   return 0;
-}
-
-int clipnce_finish_slots(const float* slots, int n_slots, const void* x, int dtype, const void* x_orig, int in_dtype,
-                         const float* rinv, const float* grad_scale, int64_t n, int64_t d, void* dx, int out_dtype,
-                         void* stream) {
-  if (!slots || !x || !x_orig || !rinv || !dx || n < 1 || d < 1 || n_slots < 1) return fail(CLIPNCE_EINVAL, "finish_slots: bad argument");
-  if (dtype != CLIPNCE_BF16 || d % 4 != 0 || sizeof(float) * 8 * (size_t)d > 48 * 1024)
-    return fail(CLIPNCE_EUNSUPPORTED, "finish_slots: bf16 compute rows, d %% 4 == 0, d <= 1536");
-  if ((in_dtype != CLIPNCE_BF16 && in_dtype != CLIPNCE_F32) || (out_dtype != CLIPNCE_BF16 && out_dtype != CLIPNCE_F32))
-    return fail(CLIPNCE_EINVAL, "finish_slots: bad dtype");
-  return launch_finish(slots, n_slots, n * d, x, x_orig, in_dtype, rinv, grad_scale, n, d, dx, out_dtype, nullptr, as_stream(stream));
 }
 
 }  // extern "C"

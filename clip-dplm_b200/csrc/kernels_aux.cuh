@@ -286,205 +286,141 @@ __global__ void rowdot_partials(const TI* __restrict__ x, const float* __restric
   if (threadIdx.x == 0) part[blockIdx.x] = ((sh[0] + sh[1]) + (sh[2] + sh[3])) + ((sh[4] + sh[5]) + (sh[6] + sh[7]));
 }
 
-// The tail of one backward side in ONE pass over the gradient (one warp per row, the row staged in shared memory):
-//   g_i   = sum over the n_split partial slabs of the column-sweep work items (fixed order; n_split = 1: the finished row)
-//   part  = sum over the block's 8 rows of rinv_i <xc_i, g_i>        (= <xhat_i, dxhat_i>: sum G.S, d logit_scale)
-//   dx_i  = rinv_i (g_i - xhat_i (xhat_i . g_i)) * grad_scale        (normalise backward; clamped rows: g_i rinv_i)
-// xc = the rows the contraction saw (compute type), xo = the caller's rows (their own type): the same pointer for bf16
-// inputs.  Replaces sum_splits + rowdot_partials + normalize_rows_bwd (three passes over [n,d] fp32).
-template <typename TC, typename TI, typename TO>
-__global__ void finish_rows(const float* __restrict__ parts, int n_split, int64_t slab, const TC* __restrict__ xc,
-                            const TI* __restrict__ xo, const float* __restrict__ rinv,
-                            const float* __restrict__ grad_scale, int64_t n, int d, TO* __restrict__ dx,
-                            float* __restrict__ ds_part) {
-  extern __shared__ float g_sh[];   // [8][d]
-  __shared__ float dot_sh[8];
+// Loads and stores of VEC consecutive elements as floats: 16-byte accesses for VEC = 4 (fp32) and 8-byte ones for bf16.
+template <int VEC, typename T>
+__device__ __forceinline__ void ldv(const T* p, float (&v)[VEC]) {
+  if constexpr (VEC == 1) {
+    v[0] = ld_f(p);
+  } else if constexpr (sizeof(T) == 4) {
+    const float4 f = *reinterpret_cast<const float4*>(p);
+    v[0] = f.x; v[1] = f.y; v[2] = f.z; v[3] = f.w;
+  } else {
+    const uint2 u = *reinterpret_cast<const uint2*>(p);
+    const float2 a = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u.x));
+    const float2 b = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u.y));
+    v[0] = a.x; v[1] = a.y; v[2] = b.x; v[3] = b.y;
+  }
+}
+template <int VEC, typename T>
+__device__ __forceinline__ void stv(T* p, const float (&v)[VEC]) {
+  if constexpr (VEC == 1) {
+    st_f(p, v[0]);
+  } else if constexpr (sizeof(T) == 4) {
+    *reinterpret_cast<float4*>(p) = make_float4(v[0], v[1], v[2], v[3]);
+  } else {
+    const __nv_bfloat162 a = __floats2bfloat162_rn(v[0], v[1]), b = __floats2bfloat162_rn(v[2], v[3]);
+    uint2 u;
+    u.x = *reinterpret_cast<const uint32_t*>(&a);
+    u.y = *reinterpret_cast<const uint32_t*>(&b);
+    *reinterpret_cast<uint2*>(p) = u;
+  }
+}
+
+// One output side of the finishing pass.  Its gradient g_i is the sum of the slabs of every contribution, each split into
+// n_split slabs `slab` elements apart: one contribution for a plain side (the split partials of a column sweep, the
+// segments of the two-sided sweep, the ranks' slots), one per virtual problem in which a group member was the resident
+// operand.  parts[] are indexed by the side's row, xc / xo / rinv / dx by row0 + that row.
+constexpr int FINISH_SIDES = 4, FINISH_CONTRIB = 8;
+struct FinishSide {
+  const float* parts[FINISH_CONTRIB];
+  int n_contrib, n_split;
+  int64_t slab;
+  int64_t row0, n;     // first row in xc / xo / rinv / dx, valid rows
+  const void* xc;      // the rows the contraction saw (compute type)
+  const void* xo;      // the caller's rows (their own type): the same pointer for rows of the compute type
+  const float* rinv;
+  void* dx;
+  float* ds_part;      // [gridDim.x] block sums of the row dots, or null
+  float* sq_part;      // [gridDim.x] block sums of |dx_i|^2, or null
+};
+struct FinishSides {
+  FinishSide s[FINISH_SIDES];
+};
+
+// The tail of a backward side in ONE pass over the fp32 gradient of the normalised rows (one warp per row, the row staged
+// in shared memory; blockIdx.y = side):
+//   g_i     = sum of the side's slabs (contribution-major, then split-major; fixed order)
+//   ds_part = sum over the block's 8 rows of rinv_i <xc_i, g_i>      (= <xhat_i, dxhat_i>: sum G.S, d logit_scale)
+//   dx_i    = rinv_i (g_i - xhat_i (xhat_i . g_i)) * grad_scale      (normalise backward; clamped rows: g_i rinv_i)
+//   sq_part = sum over the block's 8 rows of |dx_i|^2                 (the embeddings' share of a gradient norm)
+// Replaces sum_splits + rowdot_partials + normalize_rows_bwd (three passes over [n,d] fp32).  VEC = 4 (d % 4 == 0, every
+// row base 4-element aligned): every lane owns four consecutive features per 128-feature stripe, with 16-byte accesses;
+// VEC = 1: one feature per 32.  The slabs are added into the row's shared-memory copy one slab at a time, so that a lane's
+// loads of a slab are independent of each other -- memory-level parallelism is what this pass lives on.  Every lane
+// re-reads only what it wrote: no barrier needed.  grad_scale may be null (1).
+template <typename TC, typename TI, typename TO, int VEC>
+__global__ void finish_rows(const __grid_constant__ FinishSides sides, const float* __restrict__ grad_scale, int d) {
+  const FinishSide& s = sides.s[blockIdx.y];
+  extern __shared__ __align__(16) float g_sh[];   // [8][d]
+  __shared__ float dot_sh[8], sq_sh[8];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const int64_t row = (int64_t)blockIdx.x * 8 + w;
+  const int64_t r = (int64_t)blockIdx.x * 8 + w;   // row within the side
   float* g = g_sh + (size_t)w * d;
-  float dot_c = 0.f;
-  if (row < n) {
-    const float ri = rinv[row];
+  float dot_c = 0.f, sq = 0.f;
+  if (r < s.n) {
+    const int64_t row = s.row0 + r;
+    const float ri = s.rinv[row];
     const float gs = grad_scale ? grad_scale[0] : 1.f;
-    const float* pr = parts + row * d;
-    const TC* xcr = xc + row * d;
-    const TI* xor_ = xo + row * d;
-    const bool same = reinterpret_cast<const void*>(xc) == reinterpret_cast<const void*>(xo);
+    const TC* xcr = static_cast<const TC*>(s.xc) + row * d;
+    const TI* xor_ = static_cast<const TI*>(s.xo) + row * d;
+    const bool same = s.xc == s.xo;
     float dot_o = 0.f;
-    for (int k = lane; k < d; k += 32) {
-      float acc = pr[k];
-      for (int s = 1; s < n_split; ++s) acc += pr[(int64_t)s * slab + k];
-      g[k] = acc;
-      const float vc = ld_f(xcr + k);
-      dot_c = fmaf(vc, acc, dot_c);
-      if (!same) dot_o = fmaf(ld_f(xor_ + k), acc, dot_o);
-    }
-    dot_c = warp_sum(dot_c) * ri;
-    dot_o = same ? dot_c : warp_sum(dot_o) * ri;
-    const bool clamped = ri >= 0.5f / kNormEps;
-    if (clamped) dot_o = 0.f;
-    __syncwarp();
-    for (int k = lane; k < d; k += 32) {
-      const float xh = ld_f(xor_ + k) * ri;
-      st_f(dx + row * d + k, (g[k] - xh * dot_o) * (ri * gs));
-    }
-  }
-  if (ds_part != nullptr) {
-    if (lane == 0) dot_sh[w] = dot_c;
-    __syncthreads();
-    if (threadIdx.x == 0)
-      ds_part[blockIdx.x] = ((dot_sh[0] + dot_sh[1]) + (dot_sh[2] + dot_sh[3])) + ((dot_sh[4] + dot_sh[5]) + (dot_sh[6] + dot_sh[7]));
-  }
-}
-
-// four consecutive elements (4-element aligned) as floats / from floats
-template <typename T> __device__ __forceinline__ float4 ld4_f(const T* p);
-template <> __device__ __forceinline__ float4 ld4_f<float>(const float* p) { return *reinterpret_cast<const float4*>(p); }
-template <> __device__ __forceinline__ float4 ld4_f<__nv_bfloat16>(const __nv_bfloat16* p) {
-  const uint2 u = *reinterpret_cast<const uint2*>(p);
-  const float2 a = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u.x));
-  const float2 b = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u.y));
-  return make_float4(a.x, a.y, b.x, b.y);
-}
-template <typename T> __device__ __forceinline__ void st4_f(T* p, float4 v);
-template <> __device__ __forceinline__ void st4_f<float>(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
-template <> __device__ __forceinline__ void st4_f<__nv_bfloat16>(__nv_bfloat16* p, float4 v) {
-  const __nv_bfloat162 a = __floats2bfloat162_rn(v.x, v.y), b = __floats2bfloat162_rn(v.z, v.w);
-  uint2 u;
-  u.x = *reinterpret_cast<const uint32_t*>(&a);
-  u.y = *reinterpret_cast<const uint32_t*>(&b);
-  *reinterpret_cast<uint2*>(p) = u;
-}
-
-// finish_rows with 16-byte accesses (d % 4 == 0, all row bases 4-element aligned): every lane owns four consecutive
-// features per 128-feature stripe; the n_split partial rows are independent 16-byte loads (memory-level parallelism is
-// what this pass lives on: at n_split = 8 the scalar version took 52 us for 8192 x 512 against 25 us of sum_splits alone).
-template <typename TC, typename TI, typename TO>
-__global__ void finish_rows_v4(const float* __restrict__ parts, int n_split, int64_t slab, const TC* __restrict__ xc,
-                               const TI* __restrict__ xo, const float* __restrict__ rinv,
-                               const float* __restrict__ grad_scale, int64_t n, int d, TO* __restrict__ dx,
-                               float* __restrict__ ds_part) {
-  extern __shared__ __align__(16) float g4_sh[];   // [8][d]
-  __shared__ float dot_sh[8];
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const int64_t row = (int64_t)blockIdx.x * 8 + w;
-  float* g = g4_sh + (size_t)w * d;
-  float dot_c = 0.f;
-  if (row < n) {
-    const float ri = rinv[row];
-    const float gs = grad_scale ? grad_scale[0] : 1.f;
-    const float* pr = parts + row * d;
-    const TC* xcr = xc + row * d;
-    const TI* xor_ = xo + row * d;
-    const bool same = reinterpret_cast<const void*>(xc) == reinterpret_cast<const void*>(xo);
-    float dot_o = 0.f;
-    for (int k = lane * 4; k < d; k += 128) {
-      float4 acc = ld4_f(pr + k);
-#pragma unroll 4
-      for (int s = 1; s < n_split; ++s) {
-        const float4 v = ld4_f(pr + (int64_t)s * slab + k);
-        acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+    // g = the side's slabs summed contribution-major, then split-major (fixed order), accumulated in shared memory
+    const int n_slabs = s.n_contrib * s.n_split;
+    for (int t = 0; t < n_slabs; ++t) {
+      const float* pr = s.parts[t / s.n_split] + (int64_t)(t % s.n_split) * s.slab + r * d;
+      for (int k = lane * VEC; k < d; k += 32 * VEC) {
+        float v[VEC];
+        ldv(pr + k, v);
+        if (t > 0) {
+          float acc[VEC];
+          ldv(g + k, acc);
+#pragma unroll
+          for (int j = 0; j < VEC; ++j) v[j] = acc[j] + v[j];
+        }
+        stv(g + k, v);
       }
-      *reinterpret_cast<float4*>(g + k) = acc;
-      const float4 vc = ld4_f(xcr + k);
-      dot_c = fmaf(vc.x, acc.x, dot_c); dot_c = fmaf(vc.y, acc.y, dot_c);
-      dot_c = fmaf(vc.z, acc.z, dot_c); dot_c = fmaf(vc.w, acc.w, dot_c);
+    }
+    for (int k = lane * VEC; k < d; k += 32 * VEC) {
+      float acc[VEC] = {};   // a group member that is resident in no problem has no slabs: g = 0
+      if (n_slabs > 0) ldv(g + k, acc);
+      else stv(g + k, acc);
+      float vc[VEC];
+      ldv(xcr + k, vc);
+#pragma unroll
+      for (int j = 0; j < VEC; ++j) dot_c = fmaf(vc[j], acc[j], dot_c);
       if (!same) {
-        const float4 vo = ld4_f(xor_ + k);
-        dot_o = fmaf(vo.x, acc.x, dot_o); dot_o = fmaf(vo.y, acc.y, dot_o);
-        dot_o = fmaf(vo.z, acc.z, dot_o); dot_o = fmaf(vo.w, acc.w, dot_o);
+        float vo[VEC];
+        ldv(xor_ + k, vo);
+#pragma unroll
+        for (int j = 0; j < VEC; ++j) dot_o = fmaf(vo[j], acc[j], dot_o);
       }
     }
     dot_c = warp_sum(dot_c) * ri;
     dot_o = same ? dot_c : warp_sum(dot_o) * ri;
     if (ri >= 0.5f / kNormEps) dot_o = 0.f;   // clamped row: dx = g * rinv
     const float k2 = ri * gs;
-    for (int k = lane * 4; k < d; k += 128) {   // every lane re-reads only what it wrote: no barrier needed
-      const float4 gv = *reinterpret_cast<const float4*>(g + k);
-      const float4 xv = ld4_f(xor_ + k);
-      float4 o;
-      o.x = (gv.x - xv.x * ri * dot_o) * k2;
-      o.y = (gv.y - xv.y * ri * dot_o) * k2;
-      o.z = (gv.z - xv.z * ri * dot_o) * k2;
-      o.w = (gv.w - xv.w * ri * dot_o) * k2;
-      st4_f(dx + row * d + k, o);
-    }
-  }
-  if (ds_part != nullptr) {
-    if (lane == 0) dot_sh[w] = dot_c;
-    __syncthreads();
-    if (threadIdx.x == 0)
-      ds_part[blockIdx.x] = ((dot_sh[0] + dot_sh[1]) + (dot_sh[2] + dot_sh[3])) + ((dot_sh[4] + dot_sh[5]) + (dot_sh[6] + dot_sh[7]));
-  }
-}
-
-// Two finish_rows_v4 passes in ONE launch (blockIdx.y = side): the tails of the row-sharded two-sided backward -- side 0 sums
-// the segment slabs of dA_hat, side 1 the ranks' slots of dB_hat -- share the GPU instead of queueing behind each other.
-struct FinishSide {
-  const float* parts;
-  int n_split;
-  int64_t slab;
-  const void* xc;
-  const void* xo;
-  const float* rinv;
-  void* dx;
-  float* ds_part;
-};
-template <typename TC, typename TI, typename TO>
-__global__ void finish_rows_v4_dual(FinishSide s0, FinishSide s1, const float* __restrict__ grad_scale, int64_t n, int d) {
-  const FinishSide& s = blockIdx.y == 0 ? s0 : s1;
-  extern __shared__ __align__(16) float g4_sh[];   // [8][d]
-  __shared__ float dot_sh[8];
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const int64_t row = (int64_t)blockIdx.x * 8 + w;
-  float* g = g4_sh + (size_t)w * d;
-  float dot_c = 0.f;
-  if (row < n) {
-    const float ri = s.rinv[row];
-    const float gs = grad_scale ? grad_scale[0] : 1.f;
-    const float* pr = s.parts + row * d;
-    const TC* xcr = reinterpret_cast<const TC*>(s.xc) + row * d;
-    const TI* xor_ = reinterpret_cast<const TI*>(s.xo) + row * d;
-    const bool same = s.xc == s.xo;
-    float dot_o = 0.f;
-    for (int k = lane * 4; k < d; k += 128) {
-      float4 acc = ld4_f(pr + k);
-#pragma unroll 4
-      for (int q = 1; q < s.n_split; ++q) {
-        const float4 v = ld4_f(pr + (int64_t)q * s.slab + k);
-        acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+    TO* out = static_cast<TO*>(s.dx) + row * d;
+    for (int k = lane * VEC; k < d; k += 32 * VEC) {
+      float gv[VEC], xv[VEC], o[VEC];
+      ldv(g + k, gv);
+      ldv(xor_ + k, xv);
+#pragma unroll
+      for (int j = 0; j < VEC; ++j) {
+        o[j] = (gv[j] - xv[j] * ri * dot_o) * k2;
+        sq = fmaf(o[j], o[j], sq);
       }
-      *reinterpret_cast<float4*>(g + k) = acc;
-      const float4 vc = ld4_f(xcr + k);
-      dot_c = fmaf(vc.x, acc.x, dot_c); dot_c = fmaf(vc.y, acc.y, dot_c);
-      dot_c = fmaf(vc.z, acc.z, dot_c); dot_c = fmaf(vc.w, acc.w, dot_c);
-      if (!same) {
-        const float4 vo = ld4_f(xor_ + k);
-        dot_o = fmaf(vo.x, acc.x, dot_o); dot_o = fmaf(vo.y, acc.y, dot_o);
-        dot_o = fmaf(vo.z, acc.z, dot_o); dot_o = fmaf(vo.w, acc.w, dot_o);
-      }
+      stv(out + k, o);
     }
-    dot_c = warp_sum(dot_c) * ri;
-    dot_o = same ? dot_c : warp_sum(dot_o) * ri;
-    if (ri >= 0.5f / kNormEps) dot_o = 0.f;
-    const float k2 = ri * gs;
-    TO* out = reinterpret_cast<TO*>(s.dx);
-    for (int k = lane * 4; k < d; k += 128) {
-      const float4 gv = *reinterpret_cast<const float4*>(g + k);
-      const float4 xv = ld4_f(xor_ + k);
-      float4 o;
-      o.x = (gv.x - xv.x * ri * dot_o) * k2;
-      o.y = (gv.y - xv.y * ri * dot_o) * k2;
-      o.z = (gv.z - xv.z * ri * dot_o) * k2;
-      o.w = (gv.w - xv.w * ri * dot_o) * k2;
-      st4_f(out + row * d + k, o);
-    }
+    sq = warp_sum(sq);
   }
-  if (s.ds_part != nullptr) {
-    if (lane == 0) dot_sh[w] = dot_c;
+  if (s.ds_part != nullptr || s.sq_part != nullptr) {
+    if (lane == 0) { dot_sh[w] = dot_c; sq_sh[w] = sq; }
     __syncthreads();
-    if (threadIdx.x == 0)
+    if (threadIdx.x == 0 && s.ds_part != nullptr)
       s.ds_part[blockIdx.x] = ((dot_sh[0] + dot_sh[1]) + (dot_sh[2] + dot_sh[3])) + ((dot_sh[4] + dot_sh[5]) + (dot_sh[6] + dot_sh[7]));
+    if (threadIdx.x == 0 && s.sq_part != nullptr)
+      s.sq_part[blockIdx.x] = ((sq_sh[0] + sq_sh[1]) + (sq_sh[2] + sq_sh[3])) + ((sq_sh[4] + sq_sh[5]) + (sq_sh[6] + sq_sh[7]));
   }
 }
 
@@ -532,81 +468,6 @@ __global__ void loss_reduce_group(const float* __restrict__ stat_m, const float*
     __syncthreads();
   }
   if (threadIdx.x == 0) loss[n_prob] = (float)total;
-}
-
-// finish_rows_v4 for the stacked members of a group: the gradient of member m's normalised rows is the sum of the slabs of
-// every virtual problem in which m was the resident operand (its X sides and its Y sides), times the splits -- summed here
-// in fixed order, followed by the row dots and the normalise backward as in finish_rows.  grid = (ceil(n_pad / 8), members).
-//   ds_part[m][block] = sum over the block's rows of <xhat_i, g_i>   (every pair's sum G.S appears once per side: halve)
-//   sq_part[m][block] = sum over the block's rows of |dx_i|^2        (the embeddings' share of a gradient norm)
-constexpr int FG_MEMBERS = 4, FG_CONTRIB = 8;
-struct FinishGroup {
-  int n_contrib[FG_MEMBERS];
-  int vprob[FG_MEMBERS][FG_CONTRIB];   // virtual problems whose resident rows are member m
-  long long n_pad, n_valid;
-};
-template <typename TC, typename TI, typename TO>
-__global__ void finish_rows_group(const float* __restrict__ parts, int n_split, int64_t slab, FinishGroup fg,
-                                  const TC* __restrict__ xc, const TI* __restrict__ xo, const float* __restrict__ rinv,
-                                  int d, TO* __restrict__ dx, float* __restrict__ ds_part, float* __restrict__ sq_part) {
-  extern __shared__ __align__(16) float g4_sh[];   // [8][d]
-  __shared__ float dot_sh[8], sq_sh[8];
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const int m = blockIdx.y;
-  const int64_t row_m = (int64_t)blockIdx.x * 8 + w;       // row within the member
-  const int64_t row = (int64_t)m * fg.n_pad + row_m;       // stack row
-  float* g = g4_sh + (size_t)w * d;
-  float dot_c = 0.f, sq = 0.f;
-  if (row_m < fg.n_valid) {
-    const float ri = rinv[row];
-    const TC* xcr = xc + row * d;
-    const TI* xor_ = xo + row * d;
-    const bool same = reinterpret_cast<const void*>(xc) == reinterpret_cast<const void*>(xo);
-    const int nc = fg.n_contrib[m];
-    float dot_o = 0.f;
-    for (int k = lane * 4; k < d; k += 128) {
-      float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-      for (int c = 0; c < nc; ++c) {
-        const float* pr = parts + ((int64_t)fg.vprob[m][c] * fg.n_pad + row_m) * d + k;
-#pragma unroll 4
-        for (int s = 0; s < n_split; ++s) {
-          const float4 v = ld4_f(pr + (int64_t)s * slab);
-          acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
-        }
-      }
-      *reinterpret_cast<float4*>(g + k) = acc;
-      const float4 vc = ld4_f(xcr + k);
-      dot_c = fmaf(vc.x, acc.x, dot_c); dot_c = fmaf(vc.y, acc.y, dot_c);
-      dot_c = fmaf(vc.z, acc.z, dot_c); dot_c = fmaf(vc.w, acc.w, dot_c);
-      if (!same) {
-        const float4 vo = ld4_f(xor_ + k);
-        dot_o = fmaf(vo.x, acc.x, dot_o); dot_o = fmaf(vo.y, acc.y, dot_o);
-        dot_o = fmaf(vo.z, acc.z, dot_o); dot_o = fmaf(vo.w, acc.w, dot_o);
-      }
-    }
-    dot_c = warp_sum(dot_c) * ri;
-    dot_o = same ? dot_c : warp_sum(dot_o) * ri;
-    if (ri >= 0.5f / kNormEps) dot_o = 0.f;
-    for (int k = lane * 4; k < d; k += 128) {
-      const float4 gv = *reinterpret_cast<const float4*>(g + k);
-      const float4 xv = ld4_f(xor_ + k);
-      float4 o;
-      o.x = (gv.x - xv.x * ri * dot_o) * ri;
-      o.y = (gv.y - xv.y * ri * dot_o) * ri;
-      o.z = (gv.z - xv.z * ri * dot_o) * ri;
-      o.w = (gv.w - xv.w * ri * dot_o) * ri;
-      sq = fmaf(o.x, o.x, sq); sq = fmaf(o.y, o.y, sq); sq = fmaf(o.z, o.z, sq); sq = fmaf(o.w, o.w, sq);
-      st4_f(dx + row * d + k, o);
-    }
-    sq = warp_sum(sq);
-  }
-  if (lane == 0) { dot_sh[w] = dot_c; sq_sh[w] = sq; }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const int64_t o = (int64_t)m * gridDim.x + blockIdx.x;
-    ds_part[o] = ((dot_sh[0] + dot_sh[1]) + (dot_sh[2] + dot_sh[3])) + ((dot_sh[4] + dot_sh[5]) + (dot_sh[6] + dot_sh[7]));
-    sq_part[o] = ((sq_sh[0] + sq_sh[1]) + (sq_sh[2] + sq_sh[3])) + ((sq_sh[4] + sq_sh[5]) + (sq_sh[6] + sq_sh[7]));
-  }
 }
 
 // block 0: *d_scale_sum += 0.5 sum ds_part[all];  block 1 + m: sumsq[m] = sum sq_part[m][:]   (fp64, fixed-order tree)

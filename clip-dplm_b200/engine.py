@@ -220,68 +220,40 @@ class CudaEngine:
         return dx, dy, ds
 
     @_guard
-    def backward_both_sharded(self, x, y, rinv_x, rinv_y, diag_offset, scale, row_m, row_w, col_m, col_w, diag_w, x_orig,
-                              out_dtype, peers, world, rank, slots_off, grad_scale=None, flags=0, want_dscale=True,
-                              scale_dev=None):
-        """Row-sharded two-sided backward (clipnce_backward_both_sharded): -> dx [n,d] (finished), d_scale_sum [1] or None;
-        the partial dB of every owner rank is stored into its slot over NVLink peer memory (publish with a barrier, then
-        `finish_slots`)."""
-        n, d = x.shape
-        n_cols = y.shape[0]
-        dev = x.device
-        self._chk(x_orig, (torch.bfloat16, torch.float32), "x_orig")
-        ws = self._both_ws(n, n_cols, d, x.dtype, scale, flags, world, dev)
-        dx = torch.empty((n, d), dtype=out_dtype, device=dev)
-        ds = torch.zeros(1, dtype=torch.float32, device=dev) if want_dscale else None
-        xo = x if x_orig.dtype == x.dtype else x_orig
-        _lib.check(self.lib.clipnce_backward_both_sharded(_p(x), _p(y), _p(rinv_x), _p(rinv_y), n, n_cols, d, int(diag_offset),
-                                                          float(scale), _p(scale_dev), _p(row_m), _p(row_w), _p(col_m), _p(col_w),
-                                                          float(diag_w), _DT[x.dtype], flags, _p(xo), _DT[xo.dtype],
-                                                          _p(grad_scale), _p(dx), _DT[out_dtype], _p(ds), peers, world, rank,
-                                                          int(slots_off), _p(ws), ws.numel(), _stream()), "backward_both_sharded")
-        return dx, ds
-
-    @_guard
     def backward_both_sharded_sweep(self, x, y, rinv_x, rinv_y, diag_offset, scale, row_m, row_w, col_m, col_w, diag_w, peers,
                                     world, rank, slots_off, flags=0, scale_dev=None):
-        """The sweep of `backward_both_sharded` alone: dA_hat stays in the workspace as segment slabs, the partial dB_hat goes
-        to the owners' slots; finish both sides behind the barrier with `finish_sharded`."""
+        """Row-sharded two-sided backward sweep (clipnce_backward_both_sharded): dA_hat stays in the workspace as segment
+        slabs, the partial dB_hat of every owner rank is stored into its slot over NVLink peer memory; publish with a
+        barrier, then finish both sides with `finish_sharded`."""
         n, d = x.shape
         n_cols = y.shape[0]
         ws = self._both_ws(n, n_cols, d, x.dtype, scale, flags, world, x.device)
         _lib.check(self.lib.clipnce_backward_both_sharded(_p(x), _p(y), _p(rinv_x), _p(rinv_y), n, n_cols, d, int(diag_offset),
                                                           float(scale), _p(scale_dev), _p(row_m), _p(row_w), _p(col_m), _p(col_w),
-                                                          float(diag_w), _DT[x.dtype], flags, _p(x), _DT[x.dtype], None, None,
-                                                          _DT[x.dtype], None, peers, world, rank, int(slots_off), _p(ws),
-                                                          ws.numel(), _stream()), "backward_both_sharded")
+                                                          float(diag_w), _DT[x.dtype], flags, peers, world, rank, int(slots_off),
+                                                          _p(ws), ws.numel(), _stream()), "backward_both_sharded")
 
     @_guard
-    def finish_sharded(self, x, x_orig, rinv_x, y_local, y_orig, rinv_y_local, slots, n_cols, scale, world, out_dtype,
-                       grad_scale=None, flags=0, want_dscale=True):
-        """Both tails of the row-sharded two-sided backward in one launch -> dx, dy [n,d] in ``out_dtype``, d_scale_sum."""
+    def finish_sharded(self, x, x_orig, rinv_x, y_local, y_orig, rinv_y_local, slots, n_cols, scale, world, out_dtype_x,
+                       out_dtype_y, grad_scale=None, flags=0, want_dscale=True):
+        """Both tails of the row-sharded two-sided backward -> dx [n,d] in ``out_dtype_x``, dy [n,d] in ``out_dtype_y``
+        (gradients of the caller's rows x_orig / y_orig), d_scale_sum [1] f32 (or None).  One launch when both sides have
+        the same types."""
         n, d = x.shape
         dev = x.device
+        self._chk(x_orig, (torch.bfloat16, torch.float32), "x_orig")
+        self._chk(y_orig, (torch.bfloat16, torch.float32), "y_orig")
         ws = self._both_ws(n, n_cols, d, x.dtype, scale, flags, world, dev)
-        dx = torch.empty((n, d), dtype=out_dtype, device=dev)
-        dy = torch.empty((n, d), dtype=out_dtype, device=dev)
+        dx = torch.empty((n, d), dtype=out_dtype_x, device=dev)
+        dy = torch.empty((n, d), dtype=out_dtype_y, device=dev)
         ds = torch.zeros(1, dtype=torch.float32, device=dev) if want_dscale else None
         xo = x if x_orig.dtype == x.dtype else x_orig
         yo = y_local if y_orig.dtype == y_local.dtype else y_orig
         _lib.check(self.lib.clipnce_finish_sharded(_p(x), _p(xo), _p(rinv_x), _p(dx), _p(y_local), _p(yo), _p(rinv_y_local), _p(dy),
                                                    _p(slots), n, n_cols, d, _DT[x.dtype], float(scale), flags, world, _DT[xo.dtype],
-                                                   _DT[out_dtype], _p(grad_scale), _p(ds), _p(ws), ws.numel(), _stream()),
-                   "finish_sharded")
+                                                   _DT[out_dtype_x], _DT[yo.dtype], _DT[out_dtype_y], _p(grad_scale), _p(ds),
+                                                   _p(ws), ws.numel(), _stream()), "finish_sharded")
         return dx, dy, ds
-
-    @_guard
-    def finish_slots(self, slots, n_slots, x, x_orig, rinv, out_dtype, grad_scale=None):
-        """dx = normalise-backward(sum of the n_slots partial gradients [n_slots][n,d] f32), fixed order."""
-        n, d = x.shape
-        dx = torch.empty((n, d), dtype=out_dtype, device=x.device)
-        xo = x if x_orig.dtype == x.dtype else x_orig
-        _lib.check(self.lib.clipnce_finish_slots(_p(slots), n_slots, _p(x), _DT[x.dtype], _p(xo), _DT[xo.dtype], _p(rinv),
-                                                 _p(grad_scale), n, d, _p(dx), _DT[out_dtype], _stream()), "finish_slots")
-        return dx
 
     # ------------------------------------------------------------------ several pair problems in one launch
     def group_bytes(self, n_members, n_prob, n, d, dtype, scale, flags=0):

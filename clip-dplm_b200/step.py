@@ -107,7 +107,7 @@ def contrastive_forward(engine, a, b, scale, *, symmetric=True, extra=None, grou
         if need_grad:
             # two-sided backward over peer memory (one sweep emits dA and the reduce-scattered dB): nothing to gather
             both_sharded = bool(symmetric and extra is None and compute_dtype == torch.bfloat16 and
-                                getattr(xchg, "kind", "") == "nvlink-peer" and hasattr(engine, "backward_both_sharded") and
+                                getattr(xchg, "kind", "") == "nvlink-peer" and hasattr(engine, "backward_both_sharded_sweep") and
                                 engine.backward_both_bytes(n_local, n_global, d, compute_dtype, scale, flags, world) > 0)
             if not both_sharded:   # side B of the backward streams every rank's A rows; they travel behind the forward sweep
                 xchg.gather_rows_begin(a, a_c, rinv_a, compute_dtype)
@@ -194,22 +194,14 @@ def contrastive_backward(engine, st: StepState, grad_scale=None, grad_dtype_a=No
 
     if st.both_sharded:
         # row-sharded: ONE kernel sweeps local A rows x all columns, emits dA and stores every owner's partial dB straight
-        # into its slot over NVLink peer memory (contraction + reduce-scatter); after the barrier the owner sums its slots
+        # into its slot over NVLink peer memory (contraction + reduce-scatter); after the barrier the owner finishes dA from
+        # the sweep's slabs and dB from its slots
         x = st.xchg
-        same_types = st.a.dtype == st.b.dtype and (grad_dtype_a or st.a.dtype) == (grad_dtype_b or st.b.dtype)
-        if same_types and hasattr(engine, "finish_sharded"):
-            # sweep -> barrier -> ONE launch for both tails (they share the GPU instead of queueing behind each other)
-            engine.backward_both_sharded_sweep(st.a_c, st.y, st.rinv_a, st.rinv_y, off, st.scale, st.row_m, row_w, col_m, col_w,
-                                               diag_w, x.peers, x.world, x.rank, x.o_slots, st.flags, **kw)
-            x.barrier(_exchange.PHASE_GRADS)
-            da, db, ds = engine.finish_sharded(st.a_c, st.a, st.rinv_a, st.b_c, st.b, st.rinv_b, x.slots, n_glob, st.scale,
-                                               x.world, grad_dtype_a or st.a.dtype, grad_scale, st.flags)
-        else:
-            da, ds = engine.backward_both_sharded(st.a_c, st.y, st.rinv_a, st.rinv_y, off, st.scale, st.row_m, row_w, col_m,
-                                                  col_w, diag_w, st.a, grad_dtype_a or st.a.dtype, x.peers, x.world, x.rank,
-                                                  x.o_slots, grad_scale, st.flags, want_dscale=True, **kw)
-            x.barrier(_exchange.PHASE_GRADS)
-            db = engine.finish_slots(x.slots, x.world, st.b_c, st.b, st.rinv_b, grad_dtype_b or st.b.dtype, grad_scale)
+        engine.backward_both_sharded_sweep(st.a_c, st.y, st.rinv_a, st.rinv_y, off, st.scale, st.row_m, row_w, col_m, col_w,
+                                           diag_w, x.peers, x.world, x.rank, x.o_slots, st.flags, **kw)
+        x.barrier(_exchange.PHASE_GRADS)
+        da, db, ds = engine.finish_sharded(st.a_c, st.a, st.rinv_a, st.b_c, st.b, st.rinv_b, x.slots, n_glob, st.scale, x.world,
+                                           grad_dtype_a or st.a.dtype, grad_dtype_b or st.b.dtype, grad_scale, st.flags)
         ds = x.sum_scalars(ds, _exchange.PHASE_CLOSE)
         x.release()
         st.xchg = None

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define CLIPNCE_VERSION 109
+#define CLIPNCE_VERSION 110
 
 /* element types */
 #define CLIPNCE_BF16 0
@@ -201,37 +201,31 @@ int clipnce_backward_both_dx(const void* x, const void* y, const float* rinv_x, 
  * reference's all_gather formulation, old/clip_opt.py:102-112, run1/full.py:77-84): x = this rank's A rows [n_rows,d],
  * y = ALL ranks' B rows [n_cols,d] (n_cols = world * n_rows, rank r owns columns [r n_rows, (r+1) n_rows)),
  * diag_offset = rank * n_rows, row_* for the local rows, col_* for all columns.  One kernel is the contraction AND the
- * reduce-scatter of the partial dB: dx [n_rows,d] comes out finished; the partial dB_hat of the columns owned by rank s
- * is stored, as it completes, straight into rank s's buffer over NVLink peer memory at
+ * reduce-scatter of the partial dB: the segment slabs of dA_hat stay in `workspace`; the partial dB_hat of the columns
+ * owned by rank s is stored, as it completes, straight into rank s's buffer over NVLink peer memory at
  *   peer_base[s] + slots_offset + rank * n_rows * d * 4        ([world][n_rows, d] f32 slots per rank).
- * After a barrier (clipnce_link_barrier) every rank sums its world slots and applies the normalise backward with
- * clipnce_finish_slots.  peer_base: see the exchange section below.
+ * After a barrier (clipnce_link_barrier) every rank finishes both sides with clipnce_finish_sharded.  peer_base: see the
+ * exchange section below.
  */
 int clipnce_backward_both_sharded(const void* x, const void* y, const float* rinv_x, const float* rinv_y,
                                   int64_t n_rows, int64_t n_cols, int64_t d, int64_t diag_offset, float scale,
                                   const float* scale_dev,
                                   const float* row_m, const float* row_w, const float* col_m, const float* col_w,
                                   float diag_w, int dtype, int flags,
-                                  const void* x_orig, int in_dtype, const float* grad_scale, void* dx, int out_dtype,
-                                  float* d_scale_sum,
                                   void* const* peer_base, int world, int rank, int64_t slots_offset,
                                   void* workspace, size_t workspace_bytes, void* stream);
 
-/* Both tails of clipnce_backward_both_sharded in ONE launch, to be enqueued behind the barrier: call the sweep with
- * dx = NULL (its dA_hat segment slabs then stay in `workspace`, which must be the same buffer) and finish here --
- * dx = normalise-backward(sum of the slabs), dy = normalise-backward(sum of the world slots), d_scale_sum += sum G.S.
- * y_local / y_orig / rinv_y_local: this rank's B rows [n_rows,d].  Same dtype rules as clipnce_backward_dx. */
+/* Both tails of clipnce_backward_both_sharded, to be enqueued behind the barrier with the sweep's `workspace`:
+ * dx = normalise-backward(sum of the dA_hat slabs), dy = normalise-backward(sum of the world slots, in rank order),
+ * d_scale_sum += sum G.S (or NULL).  y_local / y_orig / rinv_y_local: this rank's B rows [n_rows,d].  x_orig and dx have
+ * the types x_in_dtype and x_out_dtype, y_orig and dy the types y_in_dtype and y_out_dtype, with the rules of
+ * clipnce_backward_dx.  Sides of the same types are finished in ONE launch, so that they share the GPU instead of
+ * queueing behind each other; otherwise one launch per side. */
 int clipnce_finish_sharded(const void* x, const void* x_orig, const float* rinv_x, void* dx, const void* y_local,
                            const void* y_orig, const float* rinv_y_local, void* dy, const float* slots, int64_t n_rows,
-                           int64_t n_cols, int64_t d, int dtype, float scale, int flags, int world, int in_dtype,
-                           int out_dtype, const float* grad_scale, float* d_scale_sum, void* workspace,
-                           size_t workspace_bytes, void* stream);
-
-/* dx_i = normalise-backward( sum_k slots[k][i, :] ), k < n_slots in fixed order: the tail of the row-sharded two-sided
- * backward (slots [n_slots][n, d] f32 = the ranks' partial gradients of the normalised rows x_hat). */
-int clipnce_finish_slots(const float* slots, int n_slots, const void* x, int dtype, const void* x_orig, int in_dtype,
-                         const float* rinv, const float* grad_scale, int64_t n, int64_t d, void* dx, int out_dtype,
-                         void* stream);
+                           int64_t n_cols, int64_t d, int dtype, float scale, int flags, int world, int x_in_dtype,
+                           int x_out_dtype, int y_in_dtype, int y_out_dtype, const float* grad_scale, float* d_scale_sum,
+                           void* workspace, size_t workspace_bytes, void* stream);
 
 /*
  * Several pair problems of equal shape as ONE launch per kernel: the tri-modal model, whose three symmetric InfoNCE losses

@@ -88,7 +88,7 @@ def test_library_exports_every_declared_symbol():
     lib = _lib.load()
     for name in declared:
         assert hasattr(lib, name), name
-    assert lib.clipnce_version() == 109
+    assert lib.clipnce_version() == 110
 
 
 def test_host_only_entry_points():

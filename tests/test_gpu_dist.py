@@ -15,7 +15,7 @@ from oracle import ref_step as O
 pytestmark = pytest.mark.gpu
 
 
-def _worker(rank, world, port, n, d, comm, q, both=False, ls=O.LOGIT_SCALE_INIT, mix=0.5):
+def _worker(rank, world, port, n, d, comm, q, both=False, ls=O.LOGIT_SCALE_INIT, mix=0.5, a_dtype=torch.bfloat16):
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     if both:
@@ -33,7 +33,7 @@ def _worker(rank, world, port, n, d, comm, q, both=False, ls=O.LOGIT_SCALE_INIT,
         from clip_dplm_b200 import fused_clip_loss
         a, b = O.make_inputs(n, d, seed=33, mix=mix)
         nl = n // world
-        ac = a[rank * nl:(rank + 1) * nl].cuda().bfloat16().requires_grad_(True)
+        ac = a[rank * nl:(rank + 1) * nl].cuda().to(a_dtype).requires_grad_(True)
         bc = b[rank * nl:(rank + 1) * nl].cuda().bfloat16().requires_grad_(True)
         t = torch.tensor(ls, device="cuda", requires_grad=True)
         loss = fused_clip_loss(ac, bc, t, group=dist.group.WORLD)
@@ -128,17 +128,21 @@ def _worker_topk_and_graph(rank, world, port, q):
 
 
 @pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
-@pytest.mark.parametrize("n,d,ls,mix", [(1024, 256, O.LOGIT_SCALE_INIT, 0.5), (8192, 512, O.LOGIT_SCALE_INIT, 0.5),
-                                        (4096, 512, math.log(100.0), 0.12)])
-def test_row_sharded_two_sided_backward(n, d, ls, mix):
-    """The row-sharded step through the two-sided kernel: local A rows x all columns in one sweep, dA finished locally,
-    every owner's partial dB stored into its slot over NVLink peer memory (contraction + reduce-scatter), summed in fixed
-    order -- against the sampled-row CPU oracle on the concatenated batch."""
+@pytest.mark.parametrize("n,d,ls,mix,a_dtype", [(1024, 256, O.LOGIT_SCALE_INIT, 0.5, "bfloat16"),
+                                                (8192, 512, O.LOGIT_SCALE_INIT, 0.5, "bfloat16"),
+                                                (4096, 512, math.log(100.0), 0.12, "bfloat16"),
+                                                (1024, 256, O.LOGIT_SCALE_INIT, 0.5, "float32")])
+def test_row_sharded_two_sided_backward(n, d, ls, mix, a_dtype):
+    """The row-sharded step through the two-sided kernel: local A rows x all columns in one sweep, dA finished from the
+    sweep's slabs, every owner's partial dB stored into its slot over NVLink peer memory (contraction + reduce-scatter),
+    summed in fixed order -- against the sampled-row CPU oracle on the concatenated batch."""
     import numpy as np
     from oracle import sampled as SO
     world = 2
-    # the last case runs kernel family 2 (true maxima; the clamp(max=100) regime of old/clip_opt.py:100) row-sharded
-    out = _run(_worker, (21700 + (os.getpid() % 2000), n, d, "link"), world, extra=(True, ls, mix))
+    # the third case runs kernel family 2 (true maxima; the clamp(max=100) regime of old/clip_opt.py:100) row-sharded;
+    # the last one fp32 A rows with bf16 B rows: the two sides are finished with different types
+    out = _run(_worker, (21700 + (os.getpid() % 2000), n, d, "link"), world,
+               extra=(True, ls, mix, getattr(torch, a_dtype)))
     a, b = O.make_inputs(n, d, seed=33, mix=mix)
     rng = np.random.default_rng(n)
     rows = np.sort(rng.choice(n, 128, replace=False))
