@@ -247,6 +247,8 @@ def _no_group():
 
 
 GROUP_MAX_ROWS = 8192     # measured (tools/bench_trimodal.py): 3.4x at N = 1024, 1.43x at 4096, 0.92x at 8192 against three pair steps
+GROUP_MAX_MEMBERS = 4     # aux::FINISH_SIDES: the finishing pass has one side per member
+GROUP_MAX_PROBLEMS = 4    # pair::MAX_GROUP / 2: the backward sweep runs two virtual problems per problem
 
 
 class _GroupedClipLoss(torch.autograd.Function):
@@ -325,8 +327,9 @@ def fused_clip_loss_group(members, x_member, y_member, logit_scale, *, scale_is_
     members     sequence of [N,d] CUDA embeddings of one dtype (bf16, or fp32/fp16 computed in bf16), un-normalised
     x_member / y_member   problem k pairs members[x_member[k]] (rows) with members[y_member[k]] (columns)
     Returns a [n_prob + 1] tensor (the problems' losses, then their sum), or ``None`` when the grouped launch does not
-    serve the shapes (use one `fused_clip_loss` per pair).  ``holder`` (a dict) receives ``embed_grad_sumsq`` -- the
-    squared gradient norm of every member, [n_members] f32 -- when the backward runs."""
+    serve the shapes or the counts (at most 4 members and 4 problems): then use one `fused_clip_loss` per pair.
+    ``holder`` (a dict) receives ``embed_grad_sumsq`` -- the squared gradient norm of every member, [n_members] f32 --
+    when the backward runs."""
     members = [m.to(torch.bfloat16) if m.dtype == torch.float16 else m for m in members]
     m0 = members[0]
     if m0.dim() != 2 or not m0.is_cuda:
@@ -339,6 +342,8 @@ def fused_clip_loss_group(members, x_member, y_member, logit_scale, *, scale_is_
     if m0.dtype not in (torch.bfloat16, torch.float32) or m0.shape[0] >= GROUP_MAX_ROWS:
         return None
     if _no_group():
+        return None
+    if len(members) > GROUP_MAX_MEMBERS or not 1 <= len(x_member) <= GROUP_MAX_PROBLEMS:
         return None
     if m0.dtype == torch.float32 and not (autocast_ok or torch.is_autocast_enabled()):
         return None     # fp32 rows outside autocast are computed exactly (the reference's numerics): no tensor-core group
